@@ -23,6 +23,12 @@ cores.  Prints ONE JSON line (rank 0).
              the top level.  --no-extra skips them.
   replicas_bit_identical (N > 1): checksums of the cores of all ranks after the timed steps
 
+--dump-outputs DIR (rank 0): after the timed steps, what the last of them handed its caller, as float32 .npy files:
+  tt_forward_rows.npy, a fixed seeded sample of up to 65,536 rows of the forward's output (sorted row positions
+  drawn by numpy's default_rng(0); the whole output is 105 MB at the default batch), and core<t>.npy, the cores
+  after that step's SGD update; 64 MB at most.  The inputs depend on the arguments only, so two builds can be
+  compared file by file.
+
 Timing: CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks.
 L2: four batches are rotated; one step touches 212 MB (> 126 MB L2), the rotation 850 MB.
 """
@@ -55,6 +61,8 @@ SHAPES = {
 METRIC = "TT-EmbeddingBag rows/s fwd+bwd+SGD"
 NUM_ROT = 4
 LR = 0.01   # zero-mean upstream gradient + small step: the cores stay finite over any number of steps
+DUMP_ROWS = 65536          # forward rows written by --dump-outputs
+DUMP_MAX_BYTES = 64 << 20
 
 
 def measured_peaks():
@@ -325,6 +333,21 @@ def tt_subrecord(shape_name, nnz, steps, warmup, world, rank, dev, exchange):
             "exchange_failed": failed}
 
 
+def dump_outputs(out_dir, out, cores):
+    """Writes the forward output `out` of one step (a fixed sample of its rows, as many as DUMP_MAX_BYTES leaves
+    room for beside the cores) and the `cores` after that step's update to out_dir/<name>.npy (the --dump-outputs
+    record, see the module docstring)."""
+    arrays = {"core%d" % t: c.detach().float().cpu().numpy() for t, c in enumerate(cores)}
+    out = out.reshape(-1, out.shape[-1])
+    room = DUMP_MAX_BYTES - sum(a.nbytes for a in arrays.values())
+    n = max(0, min(out.shape[0], DUMP_ROWS, room // (4 * out.shape[1])))
+    rows = np.sort(np.random.default_rng(0).choice(out.shape[0], size=n, replace=False))
+    arrays["tt_forward_rows"] = out[torch.from_numpy(rows).to(out.device)].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def replicas_identical(tensors, dev):
     """All ranks hold bit-identical copies of `tensors`? (two checksums of the bit patterns, all-gathered)"""
     import torch.distributed as dist
@@ -448,6 +471,7 @@ def run_ours(args, shape):
     # vs 0.2276 ms/step on 2 GPUs), but the process then hangs in destroy_process_group at exit
     # (measured once, 2026-10-18).  The peer-memory exchange is an ordinary kernel and captures.
     graphs, use_graph = [], ((world == 1 or xchg is not None) and not args.no_graph)
+    graph_outs = []    # graph k's forward output, rewritten by every replay of graph k
     if use_graph:
         try:
             side = torch.cuda.Stream(dev)
@@ -456,7 +480,7 @@ def run_ours(args, shape):
                 for k in range(NUM_ROT):
                     gr = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(gr, stream=side):
-                        raw_step(k)
+                        graph_outs.append(raw_step(k))
                     graphs.append(gr)
             torch.cuda.current_stream(dev).wait_stream(side)
             sync_all()
@@ -485,12 +509,20 @@ def run_ours(args, shape):
             ms = float(t.item())
         return ms
 
-    step_fn = (lambda i: graphs[i % NUM_ROT].replay()) if use_graph else (lambda i: raw_step(i % NUM_ROT))
+    eager_out = [None]
+
+    def eager_step(i):
+        eager_out[0] = raw_step(i % NUM_ROT)
+
+    step_fn = (lambda i: graphs[i % NUM_ROT].replay()) if use_graph else eager_step
     for i in range(((args.warmup + NUM_ROT - 1) // NUM_ROT) * NUM_ROT):
         step_fn(i)
     sampler = ClockSampler(local) if rank == 0 else None
     ms_total = timed(step_fn, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:     # before any later step moves the cores on
+        dump_outputs(args.dump_outputs, graph_outs[(args.steps - 1) % NUM_ROT] if use_graph else eager_out[0],
+                     cores)
     ms_step = ms_total / args.steps
     value = world * nnz / (ms_step * 1e-3)
 
@@ -826,7 +858,13 @@ def main():
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the sub-records (GraphSAGE epoch of configs 2 and 3, papers-shape step)")
     ap.add_argument("--sage-epochs", type=int, default=5, help="timed GraphSAGE epochs per sub-record (the best one counts)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU step of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     shape = SHAPES[args.shape]
