@@ -80,6 +80,11 @@ SIGNATURES = {
                                                _vp, _vp]),
     "ttg_permute_csr_workspace_bytes": (_sz, [_i64]),
     "ttg_permute_csr": (C.c_int, [_i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ttg_rcm_symmetrise_workspace_bytes": (_sz, [_i64, _i64]),
+    "ttg_rcm_symmetrise": (C.c_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp, C.POINTER(C.c_int64), _vp, _sz, _vp]),
+    "ttg_rcm_order_workspace_bytes": (_sz, [_i64]),
+    "ttg_rcm_order": (C.c_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp, C.POINTER(C.c_int64), C.POINTER(C.c_double),
+                                _vp, _sz, _vp]),
     "ttg_partition_grow": (C.c_int, [_i64, _vp, _vp, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "ttg_partition_kway": (C.c_int, [_i64, _vp, _vp, _i32, _f32, C.c_uint64, _i32, _vp, C.POINTER(C.c_int64)]),
     "ttg_sample_block_workspace_bytes": (_sz, [_i64, _i32]),

@@ -13,8 +13,9 @@
 //             stand-in for METIS-k where METIS is not available.  It is NOT METIS: the parts are
 //             connected and bounded in size, the cut is whatever the growth leaves.  The result
 //             depends on the order in which parts fill up (atomics), so only its invariants are
-//             tested.  RCMK needs no kernel: DGL calls scipy.sparse.csgraph.reverse_cuthill_mckee
-//             and so does reorder.py.
+//             tested.  RCMK: DGL calls scipy.sparse.csgraph.reverse_cuthill_mckee and so does
+//             reorder.py by default; csrc/rcm.cu computes the same permutation on the device
+//             (reorder_graph(g, "rcmk", backend="device")).
 #include <cub/device/device_scan.cuh>
 
 #include "common.cuh"

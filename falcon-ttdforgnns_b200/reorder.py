@@ -11,7 +11,11 @@
     labels_new = labels_old[perm]; train_idx_new = inverse(perm)[train_idx_old]
 
 * "rcmk" is exactly what DGL computes: scipy.sparse.csgraph.reverse_cuthill_mckee on the CSR
-  adjacency (host, offline preprocessing -- scipy is DGL's own dependency for this).
+  adjacency (host, offline preprocessing -- scipy is DGL's own dependency for this).  With
+  backend="device" the same permutation, element for element, comes from csrc/rcm.cu
+  (ttg_rcm_symmetrise / ttg_rcm_order: symmetrise, components, level-synchronous BFS on the device;
+  only numpy.argsort of the degrees runs on the host, because its tie order is part of the result):
+      new_graph, perm = reorder_graph(graph, "rcmk", backend="device")
 * "metis" is a multilevel k-way partitioner on the host (ttg_partition_kway, csrc/kway_host.cu:
   heavy-edge coarsening, grown initial parts, greedy k-way refinement), where the reference calls
   libmetis through DGL -- host code there too.  Same scheme and balance bound as METIS, not the
@@ -24,6 +28,7 @@
   oracle/reorder_oracle.py.
 """
 import ctypes as C
+import time
 from typing import Optional, Tuple
 
 import numpy as np
@@ -68,8 +73,15 @@ def permute_graph(g: CSRGraph, perm: torch.Tensor) -> CSRGraph:
     return CSRGraph(new_indptr, new_indices[:g.num_edges])
 
 
-def rcmk_permutation(g: CSRGraph) -> torch.Tensor:
-    """reverse Cuthill-McKee order, computed the way DGL's 'rcmk' does."""
+def rcmk_permutation(g: CSRGraph, backend: str = "host", stats: Optional[dict] = None) -> torch.Tensor:
+    """reverse Cuthill-McKee order, computed the way DGL's 'rcmk' does: scipy on the host
+    (backend="host") or csrc/rcm.cu (backend="device", the same permutation).  With the device
+    backend `stats`, when given, receives the seconds of each phase and the numbers of BFS levels
+    and connected components."""
+    if backend == "device":
+        return _rcmk_device(g, stats)
+    if backend != "host":
+        raise RuntimeError("rcmk_permutation: unknown backend %r (host or device)" % backend)
     from scipy import sparse
     n = g.num_nodes
     indptr = g.indptr.cpu().numpy()
@@ -77,6 +89,52 @@ def rcmk_permutation(g: CSRGraph) -> torch.Tensor:
     adj = sparse.csr_matrix((np.ones(indices.shape[0], dtype=np.int8), indices, indptr), shape=(n, n))
     perm = sparse.csgraph.reverse_cuthill_mckee(adj, symmetric_mode=False)
     return torch.from_numpy(np.ascontiguousarray(perm).astype(np.int64)).to(g.indptr.device)
+
+
+def _rcmk_device(g: CSRGraph, stats: Optional[dict]) -> torch.Tensor:
+    n, dev = g.num_nodes, g.indptr.device
+    if n == 0:
+        return torch.empty(0, dtype=torch.int64, device=dev)
+    lib = _ttg.lib()
+    with _ttg.on_device(dev):
+        t0 = time.perf_counter()
+        nnz = int(g.indptr[-1])
+        if nnz > g.num_edges:
+            raise RuntimeError("rcmk_permutation: indptr[-1] = %d > %d indices" % (nnz, g.num_edges))
+        sym_indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        sym_indices = torch.empty(max(2 * nnz, 1), dtype=torch.int32, device=dev)
+        degree = torch.empty(n, dtype=torch.int32, device=dev)
+        sym_edges = C.c_int64(0)
+        nbytes = lib.ttg_rcm_symmetrise_workspace_bytes(n, nnz)
+        if nbytes == 0:
+            raise RuntimeError("rcmk_permutation: %d nodes / %d edges out of range" % (n, nnz))
+        # ~24 bytes per symmetrised entry (7 GB at products shape): a buffer of this call alone, not the
+        # module's scratch that lives as long as the process
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        rc = lib.ttg_rcm_symmetrise(n, nnz, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(sym_indptr),
+                                    _ttg.ptr(sym_indices), _ttg.ptr(degree), C.byref(sym_edges), _ttg.ptr(ws),
+                                    ws.numel(), _ttg.stream_of(dev))
+        _ttg.check(rc, "rcm_symmetrise")
+        del ws
+        torch.cuda.current_stream(dev).synchronize()
+        t1 = time.perf_counter()
+        # scipy's own call, on the host: numpy's tie order among equal degrees is part of the result
+        rank_nodes = torch.from_numpy(np.argsort(degree.cpu().numpy())).to(dev)
+        t2 = time.perf_counter()
+        perm = torch.empty(n, dtype=torch.int64, device=dev)
+        counts = (C.c_int64 * 2)()
+        phase_ms = (C.c_double * 3)()
+        ws = torch.empty(lib.ttg_rcm_order_workspace_bytes(n), dtype=torch.uint8, device=dev)
+        rc = lib.ttg_rcm_order(n, sym_edges.value, _ttg.ptr(sym_indptr), _ttg.ptr(sym_indices), _ttg.ptr(degree),
+                               _ttg.ptr(rank_nodes), _ttg.ptr(perm), counts, phase_ms, _ttg.ptr(ws), ws.numel(),
+                               _ttg.stream_of(dev))
+        _ttg.check(rc, "rcm_order")
+    del ws
+    if stats is not None:
+        stats.update(symmetrise_s=t1 - t0, host_argsort_s=t2 - t1, components_s=phase_ms[0] / 1e3,
+                     bfs_s=phase_ms[1] / 1e3, order_s=phase_ms[2] / 1e3, levels=int(counts[0]),
+                     components=int(counts[1]), sym_edges=int(sym_edges.value))
+    return perm
 
 
 def grow_partition(g: CSRGraph, k: int, slack: float = 1.03, seed: int = 0,
@@ -153,14 +211,20 @@ def partition_permutation(labels: torch.Tensor) -> torch.Tensor:
 
 
 def reorder_graph(g: CSRGraph, algo: str, k: Optional[int] = None,
-                  nodes_perm: Optional[torch.Tensor] = None, seed: int = 0
+                  nodes_perm: Optional[torch.Tensor] = None, seed: int = 0, backend: str = "host"
                   ) -> Tuple[CSRGraph, torch.Tensor]:
+    """backend selects where "rcmk" runs ("host": scipy, "device": csrc/rcm.cu, the same order); the
+    other algorithms have one implementation each and refuse backend="device"."""
+    if backend not in ("host", "device"):
+        raise RuntimeError("reorder_graph: unknown backend %r (host or device)" % backend)
+    if backend != "host" and algo != "rcmk":
+        raise RuntimeError("reorder_graph: backend=%r applies to 'rcmk' only, not %r" % (backend, algo))
     if algo == "custom":
         if nodes_perm is None:
             raise RuntimeError("reorder_graph('custom') needs nodes_perm")
         perm = nodes_perm.to(g.indptr.device, torch.int64).contiguous()
     elif algo == "rcmk":
-        perm = rcmk_permutation(g)
+        perm = rcmk_permutation(g, backend)
     elif algo == "degree":
         perm = degree_permutation(g)
     elif algo == "grow":

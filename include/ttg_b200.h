@@ -393,6 +393,33 @@ int ttg_partition_grow(int64_t num_nodes, const int64_t* indptr, const int32_t* 
                        int32_t cap, const int64_t* seeds, int32_t sweeps, int32_t* labels_a,
                        int32_t* labels_b, int32_t* sizes, int32_t* changed, void* stream);
 
+/* ttg_rcm_symmetrise + ttg_rcm_order: reverse Cuthill-McKee on the device, element for element the
+ * permutation of scipy.sparse.csgraph.reverse_cuthill_mckee(adj, symmetric_mode=False) for adj = the CSR of
+ * in-neighbour lists (DGL's 'rcmk').  The two calls split at the one host step, numpy.argsort of the degrees
+ * (its tie order is numpy's):
+ *
+ *   ttg_rcm_symmetrise: scipy's adj + adj^T (num_edges = indptr[num_nodes]): sym_indptr int64 [n + 1],
+ *     sym_indices int32 [max(2 * num_edges, 1)] (the first *sym_edges_out entries are written), degree int32 [n]
+ *     (row length, + 1 for a self loop).  Rows are the distinct neighbours ascending when every in-list is
+ *     strictly increasing, otherwise in reverse order of first appearance in [in-list, then every v whose
+ *     in-list holds the row's node, increasing v].  *sym_edges_out is a HOST int64; the call synchronises the
+ *     stream to read it.  TTG_EINVAL also when an id lies outside [0, n) or indptr exceeds num_edges.
+ *   ttg_rcm_order: perm int64 [n] (perm[i] = old id of new node i) from the symmetrised lists, their degrees
+ *     and rank_nodes int64 [n] = numpy.argsort(degree) (device copy).  stats_out (host int64 [2], may be NULL):
+ *     {BFS levels, connected components}; phase_ms_out (host double [3], may be NULL): milliseconds spent on
+ *     {components, BFS, final order}.  Synchronises the stream once per component round and per BFS level.
+ *
+ * Out of contract: 128 or more parallel edges between one pair of nodes (scipy's int8 sum wraps and drops the
+ * entry) and in-lists of 2^31 or more entries.  Workspaces from the queries (0: sizes out of range). */
+size_t ttg_rcm_symmetrise_workspace_bytes(int64_t num_nodes, int64_t num_edges);
+int ttg_rcm_symmetrise(int64_t num_nodes, int64_t num_edges, const int64_t* indptr, const int32_t* indices,
+                       int64_t* sym_indptr, int32_t* sym_indices, int32_t* degree, int64_t* sym_edges_out,
+                       void* workspace, size_t workspace_bytes, void* stream);
+size_t ttg_rcm_order_workspace_bytes(int64_t num_nodes);
+int ttg_rcm_order(int64_t num_nodes, int64_t sym_edges, const int64_t* sym_indptr, const int32_t* sym_indices,
+                  const int32_t* degree, const int64_t* rank_nodes, int64_t* perm, int64_t* stats_out,
+                  double* phase_ms_out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ttg_partition_kway: multilevel k-way partition (heavy-edge coarsening, grown initial parts, greedy
  * k-way refinement while uncoarsening) -- the role of METIS behind dgl.reorder_graph(g, 'metis',
  * permute_config={'k': k}) and dgl.metis_partition (graphloader.py:370, 377, 440).  HOST code like
