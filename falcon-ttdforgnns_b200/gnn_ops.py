@@ -196,6 +196,60 @@ def aggregate(block: Block, x: torch.Tensor, mean: bool,
     return _SpMM.apply(block, x, mean, edge_weight)
 
 
+def mean_agg_plan(g) -> torch.Tensor:
+    """The work-item plan of ttg_mean_agg for a whole graph (sampler.CSRGraph or anything with int64 `indptr`,
+    int32 `indices`), built once and kept with the graph like Block.transposed(): every layer and width reuses
+    it.  Rebuilt if indptr is replaced or modified in place."""
+    key = (g.indptr.data_ptr(), g.indptr._version, g.indptr.numel(), g.indices.numel())
+    kept = getattr(g, "_mean_agg_plan", None)
+    if kept is not None and kept[0] == key:
+        return kept[1]
+    n, e = g.indptr.numel() - 1, g.indices.numel()
+    _ttg.require_cuda(g.indptr, "indptr", torch.int64)
+    _ttg.require_cuda(g.indices, "indices", torch.int32)
+    dev = g.indptr.device
+    lib = _ttg.lib()
+    plan_bytes = lib.ttg_mean_agg_plan_bytes(n, e)
+    ws_bytes = lib.ttg_mean_agg_workspace_bytes(n, e, 1)
+    if plan_bytes == 0 or ws_bytes == 0:
+        raise RuntimeError("mean_agg_plan: %d nodes / %d edges out of range" % (n, e))
+    with _ttg.on_device(dev):
+        plan = torch.empty(plan_bytes, dtype=torch.uint8, device=dev)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)     # the scan's scratch, for this call only
+        rc = lib.ttg_mean_agg_plan(n, e, _ttg.ptr(g.indptr), _ttg.ptr(plan), plan_bytes, _ttg.ptr(ws), ws_bytes,
+                                   _ttg.stream_of(dev))
+        _ttg.check(rc, "mean_agg_plan")
+    object.__setattr__(g, "_mean_agg_plan", (key, plan))
+    return plan
+
+
+def aggregate_full(g, x: torch.Tensor) -> torch.Tensor:
+    """out[v] = mean of x over the in-neighbours of v, for EVERY node of the graph g (zero rows for nodes without
+    in-edges); not differentiable.  For full-neighbour inference: rows are cut into work items of at most 256
+    edges (ttg_mean_agg), so a node with 40 k in-edges does not hold one warp for the whole call as it would in
+    aggregate()'s one-warp-per-destination kernel.  Deterministic: the same bits from every call."""
+    x = _ttg.require_cuda(x.contiguous(), "x", torch.float32)
+    n, e = g.indptr.numel() - 1, g.indices.numel()
+    if x.dim() != 2 or x.size(0) != n:
+        raise RuntimeError("aggregate_full: x must be [num_nodes=%d, F], got %s" % (n, tuple(x.shape)))
+    F = x.size(1)
+    dev = x.device
+    if n == 0:
+        return torch.empty((0, F), dtype=torch.float32, device=dev)
+    lib = _ttg.lib()
+    with _ttg.on_device(dev):
+        plan = mean_agg_plan(g)
+        ws_bytes = lib.ttg_mean_agg_workspace_bytes(n, e, F)
+        if ws_bytes == 0:
+            raise RuntimeError("aggregate_full: F=%d out of range" % F)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        out = torch.empty((n, F), dtype=torch.float32, device=dev)
+        rc = lib.ttg_mean_agg(n, e, F, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(plan), plan.numel(),
+                              _ttg.ptr(x), _ttg.ptr(out), _ttg.ptr(ws), ws_bytes, _ttg.stream_of(dev))
+        _ttg.check(rc, "mean_agg")
+    return out
+
+
 class SAGEConv(nn.Module):
     """GraphSAGE layer with DGL 2.1 `SAGEConv(in, out, 'mean')` semantics:
     out = fc_self(h_dst) + fc_neigh(mean_{u in N(v)} h_src[u]) + bias, the neighbour Linear being
@@ -228,13 +282,27 @@ class SAGEConv(nn.Module):
         else:
             if h_dst is None:
                 h_dst = h_src[:block.num_dst]
-            if self.in_feats > self.out_feats:
-                h_neigh = aggregate(block, self.fc_neigh(h_src), mean=True)
-            else:
-                h_neigh = self.fc_neigh(aggregate(block, h_src, mean=True))
+            h_neigh = self._neighbours(lambda h: aggregate(block, h, mean=True), h_src)
         out = self.fc_self(h_dst) + h_neigh
         if self.bias is not None:
             out = out + self.bias
+        return out
+
+    def _neighbours(self, mean_of, h_src: torch.Tensor) -> torch.Tensor:
+        """fc_neigh of the neighbour mean, `mean_of` being the aggregation: DGL applies the Linear first when
+        that shrinks the rows to gather (in_feats > out_feats), after the aggregation otherwise."""
+        if self.in_feats > self.out_feats:
+            return mean_of(self.fc_neigh(h_src))
+        return self.fc_neigh(mean_of(h_src))
+
+    @torch.no_grad()
+    def forward_full(self, g, h: torch.Tensor) -> torch.Tensor:
+        """The layer on every node of a whole graph g (sampler.CSRGraph; h [num_nodes, in_feats]): layer-wise
+        full-neighbour inference (gnn_model.py:220-253), the neighbour mean by aggregate_full."""
+        out = self.fc_self(h)
+        out += self._neighbours(lambda x: aggregate_full(g, x), h)
+        if self.bias is not None:
+            out += self.bias
         return out
 
     def forward_aggregated(self, h_dst: torch.Tensor, h_mean: torch.Tensor) -> torch.Tensor:

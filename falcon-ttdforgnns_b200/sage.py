@@ -81,6 +81,35 @@ class SAGE(nn.Module):
                 h = self.dropout(F.relu(h))
         return h
 
+    @torch.no_grad()
+    def inference(self, g: CSRGraph) -> torch.Tensor:
+        """[num_nodes, n_classes] logits of every node of g with ALL its in-neighbours, computed layer by layer
+        over the whole graph (gnn_model.py:220-253): the rows of all nodes, then each layer on every node
+        (SAGEConv.forward_full), ReLU between layers, no dropout.  The same for fuse_input on or off; the cores,
+        the dense parameters and self.training are left as they are."""
+        h = self._all_rows(g.num_nodes)
+        for l, layer in enumerate(self.layers):
+            h = layer.forward_full(g, h)
+            if l != len(self.layers) - 1:
+                h = F.relu_(h)
+        return h
+
+    def _all_rows(self, n: int) -> torch.Tensor:
+        """Input features of nodes 0 .. n - 1: the row kernel on an implicit range where the table has one
+        (ttg_tt_rows_range), else the lookup on arange(n) as the reference does (gnn_model.py:228-231)."""
+        emb = self.embed_layer
+        if n > emb.num_embeddings:
+            raise RuntimeError("SAGE.inference: the graph has %d nodes, the embedding %d rows"
+                               % (n, emb.num_embeddings))
+        dev = emb.tt_cores[0].device
+        ids = torch.arange(n, device=dev)
+        if self.embed_name == "eff":
+            return emb(ids)
+        rows = emb.rows_range(0, n)
+        if rows is not None:
+            return rows
+        return emb(ids, torch.arange(n + 1, device=dev))
+
     def _fused_first_layer(self, block: Block, input_nodes: torch.Tensor) -> torch.Tensor:
         """Bags 0 .. num_dst - 1: the destination nodes themselves; bags num_dst .. 2 num_dst - 1: their
         sampled neighbours, summed by the lookup (pooling "sum" of TTEmbeddingBag) and divided by the
@@ -94,6 +123,22 @@ class SAGE(nn.Module):
         deg = block.in_degrees().clamp(min=1).to(torch.float32)
         h_mean = out[nd:] / deg.unsqueeze(1)
         return self.layers[0].forward_aggregated(out[:nd], h_mean)
+
+
+@torch.no_grad()
+def evaluate(model: SAGE, g: CSRGraph, labels: torch.Tensor, val_nid: torch.Tensor, test_nid: torch.Tensor):
+    """(validation accuracy, test accuracy, logits of every node) of the full-neighbour inference, as the
+    reference's evaluate (sage_dgl_partition.py:366-371): eval mode, SAGE.inference, accuracy of the argmax on
+    each node set, train mode again."""
+    model.eval()
+    try:
+        pred = model.inference(g)
+    finally:
+        model.train()
+    hit = pred.argmax(1) == labels.to(pred.device)
+    val_acc = float(hit[val_nid.to(pred.device)].float().mean())
+    test_acc = float(hit[test_nid.to(pred.device)].float().mean())
+    return val_acc, test_acc, pred
 
 
 def synthetic_graph(num_nodes: int, num_edges: int, device, seed: int = 0, alpha: float = 2.1

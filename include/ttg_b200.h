@@ -316,6 +316,27 @@ int ttg_spmm_csr_bwd(int64_t num_dst, int32_t F, const int64_t* indptr,
                      const int32_t* indices, const float* edge_weight, int32_t mean,
                      const float* dout, float* dx, void* stream);
 
+/* (d-2) mean over the in-neighbours of EVERY node of a whole graph (full-neighbour inference, the
+ * layer-wise SAGE.inference of gnn_model.py:220-253), balanced by edges instead of by destinations:
+ *   out[v][:] = (1 / deg(v)) * sum_{e in [indptr[v], indptr[v+1])} x[indices[e]][:]   (0 rows: deg 0)
+ * Graph: indptr int64 [num_nodes + 1], indices int32 [num_edges] (ids < num_nodes); x, out fp32
+ * [num_nodes][F], any F >= 1 (16-byte columns when F % 4 == 0).
+ * ttg_mean_agg_plan cuts every row into work items of at most 256 edges (a per-node count, a scan, a
+ * scatter); the plan depends on indptr alone and serves every later ttg_mean_agg on the same graph, at any
+ * width.  Plan buffer: ttg_mean_agg_plan_bytes(num_nodes, num_edges) bytes, 16-byte aligned (bounded by
+ * num_nodes + num_edges / 256 items of 16 bytes).  Workspace of either call:
+ * ttg_mean_agg_workspace_bytes(num_nodes, num_edges, F) (plan build: any F >= 1); it holds the partial rows
+ * of nodes with more than 256 in-edges, which a second pass sums in item order: no float atomics, the same
+ * bits from every call.  Both queries return 0 for arguments out of range (num_nodes < 0 or >= 2^31,
+ * num_edges < 0 or > 2^37, F <= 0).  The plan must come from the same indptr. */
+size_t ttg_mean_agg_plan_bytes(int64_t num_nodes, int64_t num_edges);
+size_t ttg_mean_agg_workspace_bytes(int64_t num_nodes, int64_t num_edges, int32_t F);
+int ttg_mean_agg_plan(int64_t num_nodes, int64_t num_edges, const int64_t* indptr, void* plan,
+                      size_t plan_bytes, void* workspace, size_t workspace_bytes, void* stream);
+int ttg_mean_agg(int64_t num_nodes, int64_t num_edges, int32_t F, const int64_t* indptr,
+                 const int32_t* indices, const void* plan, size_t plan_bytes, const float* x, float* out,
+                 void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * (f-4) the sparse part of GATConv on a CSR-by-destination block.
  * replaces: apply_edges(u_add_v) + leaky_relu + edge_softmax and update_all(u_mul_e, sum) of
