@@ -91,6 +91,17 @@ SIGNATURES = {
                                 _vp, _sz, _vp]),
     "ttg_partition_grow": (C.c_int, [_i64, _vp, _vp, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "ttg_partition_kway": (C.c_int, [_i64, _vp, _vp, _i32, _f32, C.c_uint64, _i32, _vp, C.POINTER(C.c_int64)]),
+    "ttg_partition_kway_initial": (C.c_int, [_i64, _vp, _vp, _vp, _vp, _i64, _i32, _f32, C.c_uint64, _i32, _vp]),
+    "ttg_kway_symmetrise_workspace_bytes": (_sz, [_i64, _i64]),
+    "ttg_kway_symmetrise": (C.c_int, [_i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(C.c_int64), _vp, _sz, _vp]),
+    "ttg_kway_coarsen_workspace_bytes": (_sz, [_i64, _i64]),
+    "ttg_kway_coarsen": (C.c_int, [_i64, _i64, _vp, _vp, _vp, _vp, _i32, C.c_uint64, _i32, _vp, _vp, _vp, _vp, _vp,
+                                   C.POINTER(C.c_int64), _vp, _sz, _vp]),
+    "ttg_kway_refine_workspace_bytes": (_sz, [_i64, _i32]),
+    "ttg_kway_refine": (C.c_int, [_i64, _vp, _vp, _vp, _vp, _i64, _i32, _f32, _i32, C.c_uint64, _i32, _i32, _vp, _vp,
+                                  _vp, C.POINTER(C.c_int64), _vp, _sz, _vp]),
+    "ttg_kway_edge_cut_workspace_bytes": (_sz, []),
+    "ttg_kway_edge_cut": (C.c_int, [_i64, _vp, _vp, _vp, C.POINTER(C.c_int64), _vp, _sz, _vp]),
     "ttg_sample_block_workspace_bytes": (_sz, [_i64, _i32]),
     "ttg_sample_block": (C.c_int, [_i64, _vp, _vp, _i64, _vp, _i32, C.c_uint64, _vp, _vp, _vp, _vp,
                                    _vp, _sz, _vp]),

@@ -17,7 +17,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(HERE, "build")
 LIB = os.path.join(LIBDIR, "libttg_b200.so")
-SOURCES = ["api.cu", "tt_generic.cu", "tt_sorted.cu", "tt_mma.cu", "tt_tc5.cu", "tt_rmma.cu", "cache.cu", "spmm.cu", "sampler.cu", "gat.cu", "peer.cu", "reorder.cu", "rcm.cu", "kway_host.cu"]
+SOURCES = ["api.cu", "tt_generic.cu", "tt_sorted.cu", "tt_mma.cu", "tt_tc5.cu", "tt_rmma.cu", "cache.cu", "spmm.cu", "sampler.cu", "gat.cu", "peer.cu", "reorder.cu", "rcm.cu", "kway_host.cu", "kway.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "tc5.cuh"), os.path.join(HERE, "..", "include", "ttg_b200.h")]
 
 NVCC_FLAGS = [

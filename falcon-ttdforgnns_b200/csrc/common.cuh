@@ -93,6 +93,38 @@ int make_ttdev(const ttg_shape* shape, const float* const* host_core_ptrs, TTDev
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// number of bits that hold every value in [0, x] (radix-sort key widths)
+static inline int bits_for(uint64_t x) {
+  int b = 0;
+  while (b < 64 && (x >> b) != 0) ++b;
+  return b;
+}
+
+// lays a caller's workspace out in 256-byte aligned pieces; with base == nullptr it only sums the sizes
+struct Carver {
+  void* base;
+  size_t off = 0;
+  void* take(size_t bytes) {
+    char* p = base ? (char*)base + off : nullptr;
+    off += align_up(bytes, 256);
+    return (void*)p;
+  }
+};
+
+// one value from the device, waited for
+template <typename T>
+int read_back(T* host, const T* dev, cudaStream_t stream) {
+  TTG_CUDA(cudaMemcpyAsync(host, dev, sizeof(T), cudaMemcpyDeviceToHost, stream));
+  TTG_CUDA(cudaStreamSynchronize(stream));
+  return TTG_OK;
+}
+
+#define TTG_RC(expr)               \
+  do {                             \
+    const int _rc = (expr);        \
+    if (_rc != TTG_OK) return _rc; \
+  } while (0)
+
 // ---- device helpers ------------------------------------------------------------------
 __device__ __forceinline__ float4 ldg4(const float* p) {
   return __ldg(reinterpret_cast<const float4*>(p));
@@ -263,5 +295,12 @@ int r_cores(const TTDev& tt, const RPlan& pl, float* const* dcore, cudaStream_t 
 int mma_finalize_parts(const TTDev& tt, const float* d0parts, int nparts, const float* d2parts, int n2parts,
                        float* const* dcore, int32_t optim, float lr, float eps, float* const* state,
                        cudaStream_t stream);
+
+// balance bounds of the k-way partitioners (kway_host.cu): every part at most maxpw and at least minpw vertices
+// on the finest level, maxpw_coarse / minpw_coarse (1.3 x slack) on the coarser ones
+struct KwayBounds {
+  int64_t maxpw, minpw, maxpw_coarse, minpw_coarse;
+};
+void kway_bounds(int64_t num_nodes, int32_t k, float ubfactor, KwayBounds* b);
 
 }  // namespace ttg

@@ -466,7 +466,40 @@ int64_t weighted_cut(const WGraph& g, const std::vector<int32_t>& part) {
 constexpr int kInitialTrials = 8;
 constexpr double kCoarseSlack = 1.3;
 
+// a few grown partitions of the coarsest graph, each refined there with the coarse bounds; the one with the
+// smallest cut goes on (the host partitioner below and the device partitioner's host step, csrc/kway.cu)
+void initial_parts(const WGraph& cg, int32_t k, int64_t maxpw_coarse, int64_t minpw_coarse, int32_t refine_passes,
+                   Rng& rng, std::vector<int32_t>& part) {
+  int64_t best_cut = -1;
+  for (int trial = 0; trial < kInitialTrials; ++trial) {
+    std::vector<int32_t> cand;
+    initial_partition(cg, k, rng, cand);
+    Refiner r(cg, k, maxpw_coarse, minpw_coarse, cand);
+    r.balance(rng);
+    r.refine(refine_passes, rng);
+    r.balance(rng);
+    const int64_t cut = weighted_cut(cg, cand);
+    if (best_cut < 0 || cut < best_cut) {
+      best_cut = cut;
+      part.swap(cand);
+    }
+  }
+}
+
 }  // namespace
+
+void kway_bounds(int64_t num_nodes, int32_t k, float ubfactor, KwayBounds* b) {
+  const int64_t ideal = (num_nodes + k - 1) / k;
+  b->maxpw = std::max<int64_t>(ideal, (int64_t)((double)ubfactor * (double)ideal));
+  b->minpw = (int64_t)((double)(num_nodes / k) / (double)ubfactor);   // METIS keeps parts above 1/ufactor too
+  // On every level but the finest the parts may be kCoarseSlack times heavier / lighter than the bound: with the
+  // strict bound a community that the grown parts split in halves stays split (each half is balanced against the
+  // other, the part it should join is full); with slack the halves flow together and the parts that lose them
+  // take their own strays back, so the bound is met again by the time the finest level enforces it.
+  b->maxpw_coarse = (int64_t)(b->maxpw * kCoarseSlack);
+  b->minpw_coarse = (int64_t)(b->minpw / kCoarseSlack);
+}
+
 }  // namespace ttg
 
 extern "C" int ttg_partition_kway(int64_t num_nodes, const int64_t* indptr, const int32_t* indices,
@@ -516,33 +549,11 @@ extern "C" int ttg_partition_kway(int64_t num_nodes, const int64_t* indptr, cons
     cmaps.push_back(std::move(cmap));
     levels.push_back(std::move(c));
   }
-  const int64_t ideal = (num_nodes + k - 1) / k;
-  const int64_t maxpw = std::max<int64_t>(ideal, (int64_t)((double)ubfactor * (double)ideal));
-  const int64_t minpw = (int64_t)((double)(num_nodes / k) / (double)ubfactor);   // METIS keeps parts above 1/ufactor too
-  // On every level but the finest the parts may be kCoarseSlack times heavier / lighter than the bound: with the
-  // strict bound a community that the grown parts split in halves stays split (each half is balanced against the
-  // other, the part it should join is full); with slack the halves flow together and the parts that lose them
-  // take their own strays back, so the bound is met again by the time the finest level enforces it.
-  const int64_t maxpw_coarse = (int64_t)(maxpw * kCoarseSlack), minpw_coarse = (int64_t)(minpw / kCoarseSlack);
-  // a few grown partitions of the coarsest graph, each refined there; the one with the smallest cut goes on
+  KwayBounds b;
+  kway_bounds(num_nodes, k, ubfactor, &b);
+  const int64_t maxpw = b.maxpw, minpw = b.minpw, maxpw_coarse = b.maxpw_coarse, minpw_coarse = b.minpw_coarse;
   std::vector<int32_t> part;
-  {
-    const WGraph& cg = levels.back();
-    int64_t best_cut = -1;
-    for (int trial = 0; trial < kInitialTrials; ++trial) {
-      std::vector<int32_t> cand;
-      initial_partition(cg, k, rng, cand);
-      Refiner r(cg, k, maxpw_coarse, minpw_coarse, cand);
-      r.balance(rng);
-      r.refine(refine_passes, rng);
-      r.balance(rng);
-      const int64_t cut = weighted_cut(cg, cand);
-      if (best_cut < 0 || cut < best_cut) {
-        best_cut = cut;
-        part.swap(cand);
-      }
-    }
-  }
+  initial_parts(levels.back(), k, maxpw_coarse, minpw_coarse, refine_passes, rng, part);
   for (size_t lv = levels.size(); lv-- > 0;) {
     Refiner r(levels[lv], k, lv > 0 ? maxpw_coarse : maxpw, lv > 0 ? minpw_coarse : minpw, part);
     r.balance(rng);
@@ -566,6 +577,46 @@ extern "C" int ttg_partition_kway(int64_t num_nodes, const int64_t* indptr, cons
   }
   } catch (const std::exception& ex) {   // host memory (the graph is held about three times) or a worker thread
     set_error("partition_kway: %s", ex.what());
+    return TTG_ENOMEM;
+  }
+  return TTG_OK;
+}
+
+extern "C" int ttg_partition_kway_initial(int64_t num_nodes, const int64_t* xadj, const int32_t* adj,
+                                          const int32_t* adjw, const int32_t* vw, int64_t total_nodes, int32_t k,
+                                          float ubfactor, uint64_t seed, int32_t refine_passes, int32_t* part_out) {
+  using namespace ttg;
+  TTG_CHECK_ARG(num_nodes > 0 && num_nodes <= total_nodes && total_nodes < (int64_t)INT32_MAX,
+                "partition_kway_initial: %lld of %lld nodes out of range", (long long)num_nodes,
+                (long long)total_nodes);
+  TTG_CHECK_ARG(xadj != nullptr && vw != nullptr && part_out != nullptr, "partition_kway_initial: null pointer");
+  TTG_CHECK_ARG(k >= 1 && k <= total_nodes, "partition_kway_initial: k=%d for %lld nodes", k, (long long)total_nodes);
+  TTG_CHECK_ARG(ubfactor >= 1.0f, "partition_kway_initial: ubfactor %g below 1", (double)ubfactor);
+  TTG_CHECK_ARG(xadj[0] == 0, "partition_kway_initial: xadj[0] = %lld", (long long)xadj[0]);
+  for (int64_t v = 0; v < num_nodes; ++v)
+    TTG_CHECK_ARG(xadj[v + 1] >= xadj[v] && vw[v] >= 1, "partition_kway_initial: bad row or weight at vertex %lld",
+                  (long long)v);
+  const int64_t m = xadj[num_nodes];
+  TTG_CHECK_ARG(m == 0 || (adj != nullptr && adjw != nullptr), "partition_kway_initial: null adjacency");
+  for (int64_t e = 0; e < m; ++e)
+    TTG_CHECK_ARG(adj[e] >= 0 && adj[e] < num_nodes && adjw[e] >= 1,
+                  "partition_kway_initial: neighbour id %d out of range", adj[e]);
+  if (refine_passes <= 0) refine_passes = 10;
+  try {
+    WGraph g;
+    g.n = (int32_t)num_nodes;
+    g.xadj.assign(xadj, xadj + num_nodes + 1);
+    g.adj.assign(adj, adj + m);
+    g.adjw.assign(adjw, adjw + m);
+    g.vw.assign(vw, vw + num_nodes);
+    KwayBounds b;
+    kway_bounds(total_nodes, k, ubfactor, &b);
+    Rng rng(seed);
+    std::vector<int32_t> part;
+    initial_parts(g, k, b.maxpw_coarse, b.minpw_coarse, refine_passes, rng, part);
+    std::memcpy(part_out, part.data(), sizeof(int32_t) * (size_t)num_nodes);
+  } catch (const std::exception& ex) {
+    set_error("partition_kway_initial: %s", ex.what());
     return TTG_ENOMEM;
   }
   return TTG_OK;

@@ -40,13 +40,6 @@ namespace {
 
 constexpr uint32_t kFromTranspose = 0x80000000u;   // appearance rank of an adj^T entry: after the in-list
 
-// number of bits that hold every value in [0, x]
-int bits_for(uint64_t x) {
-  int b = 0;
-  while (b < 64 && (x >> b) != 0) ++b;
-  return b;
-}
-
 // ---- symmetrise ------------------------------------------------------------------------------------
 // one warp per row v of the in-lists: (v, u) with its position in the list and (u, v) ranked after every
 // in-list entry in increasing v.  A stable sort by (row, col) then keeps each pair's first appearance first.
@@ -301,16 +294,6 @@ order_reverse_kernel(int64_t n, const int32_t* __restrict__ sorted, int64_t* __r
 }
 
 // ---- workspaces ------------------------------------------------------------------------------------------
-struct Carver {
-  void* base;
-  size_t off = 0;
-  void* take(size_t bytes) {
-    char* p = base ? (char*)base + off : nullptr;
-    off += align_up(bytes, 256);
-    return (void*)p;
-  }
-};
-
 struct SymWs {
   uint64_t *keys_a, *keys_b;
   uint32_t *vals_a, *vals_b;
@@ -388,19 +371,6 @@ OrderWs carve_order(void* ws, int64_t n) {
 bool nodes_in_range(int64_t n) { return n > 0 && n < ((int64_t)1 << 31); }
 // 2 * nnz (row, col) pairs; each in-list shorter than 2^31 (appearance ranks are 31-bit)
 bool edges_in_range(int64_t nnz) { return nnz >= 0 && nnz <= ((int64_t)1 << 40); }
-
-template <typename T>
-int read_back(T* host, const T* dev, cudaStream_t stream) {
-  TTG_CUDA(cudaMemcpyAsync(host, dev, sizeof(T), cudaMemcpyDeviceToHost, stream));
-  TTG_CUDA(cudaStreamSynchronize(stream));
-  return TTG_OK;
-}
-
-#define TTG_RC(expr)            \
-  do {                          \
-    const int _rc = (expr);     \
-    if (_rc != TTG_OK) return _rc; \
-  } while (0)
 
 double ms_since(std::chrono::steady_clock::time_point t0) {
   return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();

@@ -5,6 +5,7 @@
     new_graph, perm = reorder_graph(graph, "rcmk")               # perm[i] = old id of new node i
     new_graph, perm = reorder_graph(graph, "metis", k=125)       # multilevel k-way partition, part by part
     new_graph, perm = recursive_metis_reorder(graph, [50, 60, 60])   # graphloader.py:358-372
+    new_graph, perm = reorder_graph(graph, "kway", k=125)        # multilevel k-way on the device
     new_graph, perm = reorder_graph(graph, "grow", k=125)        # label propagation on the device
     new_graph, perm = reorder_graph(graph, "custom", nodes_perm=p)
     new_graph, perm = reorder_graph(graph, "degree")             # graphloader.py:275-285: high in-degree first
@@ -21,6 +22,14 @@
   libmetis through DGL -- host code there too.  Same scheme and balance bound as METIS, not the
   same partition (METIS is not in this image; parity with its order is unpinned).  The new order
   is part by part, old order within a part (stable), as DGL's METIS reorder sorts by part id.
+* "kway" is the same multilevel scheme with its data-parallel steps on the device
+  (kway_partition_device, csrc/kway.cu: sort-based symmetrise, handshake heavy-edge matching and
+  contraction level by level, the host partitioner's grown initial parts on the coarsest graph,
+  Jet-style synchronous label propagation with an afterburner and sorted admission on the way up).
+  The same balance bounds and cut quality bar as "metis", a different partition (neither the host
+  partitioner's nor METIS'); device-only, so it takes no backend:
+      new_graph, perm = reorder_graph(graph, "kway", k=125)
+      new_graph, perm = recursive_metis_reorder(graph, [50, 60, 60], algo="kway")
 * "grow" partitions on the device (ttg_partition_grow): k connected parts of at most
   ceil(N / k * slack) nodes grown from k seed nodes drawn uniformly (seeded); nodes no part
   could take fill the parts with room.  Much faster than "metis" and a much larger cut.
@@ -191,6 +200,121 @@ def kway_partition(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int = 0, r
     return (labels, int(cut.value)) if return_cut else labels
 
 
+def kway_partition_device(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int = 0, refine_passes: int = 10,
+                          return_cut: bool = False, stats: Optional[dict] = None):
+    """int32 part id of every node from the multilevel k-way partitioner on the device (csrc/kway.cu); the
+    contract of kway_partition: every part holds at most max(ceil(N / k), ubfactor * ceil(N / k)) nodes and at
+    least floor(N / k) / ubfactor, the labels are on the graph's device and depend on the graph and the seed
+    alone; with return_cut also the number of input edges whose ends lie in different parts.  The partition
+    is not kway_partition's (nor METIS'): the matching and the refinement are parallel formulations.  Only the
+    initial parts of the coarsest graph are computed on the host, by the host partitioner's own code.  `stats`,
+    when given, receives the seconds of each phase, the number of levels and the coarsest graph's size."""
+    n, dev = g.num_nodes, g.indptr.device
+    k = int(k)
+    if not 0 < k <= max(n, 1):
+        raise RuntimeError("kway_partition_device: k=%d out of range" % k)
+    if ubfactor < 1.0:
+        raise RuntimeError("kway_partition_device: ubfactor %g below 1" % ubfactor)
+    if n == 0 or k == 1:
+        labels = torch.zeros(n, dtype=torch.int32, device=dev)
+        return (labels, 0) if return_cut else labels
+    lib = _ttg.lib()
+    stream = _ttg.stream_of(dev)
+    ub = float(ubfactor)
+    times = {}
+    with _ttg.on_device(dev):
+        sync = torch.cuda.current_stream(dev).synchronize
+        t0 = time.perf_counter()
+        nnz = int(g.indptr[-1])
+        if nnz > g.num_edges:
+            raise RuntimeError("kway_partition_device: indptr[-1] = %d > %d indices" % (nnz, g.num_edges))
+        nbytes = lib.ttg_kway_symmetrise_workspace_bytes(n, nnz)
+        if nbytes == 0:
+            raise RuntimeError("kway_partition_device: %d nodes / %d edges out of range" % (n, nnz))
+        xadj = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        adj = torch.empty(max(2 * nnz, 1), dtype=torch.int32, device=dev)
+        adjw = torch.empty(max(2 * nnz, 1), dtype=torch.int32, device=dev)
+        vw = torch.empty(n, dtype=torch.int32, device=dev)
+        m = C.c_int64(0)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)   # ~24 bytes per symmetrised entry: this call's alone
+        _ttg.check(lib.ttg_kway_symmetrise(n, nnz, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(xadj),
+                                           _ttg.ptr(adj), _ttg.ptr(adjw), _ttg.ptr(vw), C.byref(m), _ttg.ptr(ws),
+                                           ws.numel(), stream), "kway_symmetrise")
+        del ws
+        # trim the symmetrised lists to their size: every level is kept for the way back up
+        levels = [(n, m.value, xadj, adj[:m.value].clone(), adjw[:m.value].clone(), vw)]
+        del adj, adjw
+        t1 = time.perf_counter()
+        times["symmetrise_s"] = t1 - t0
+        # the host partitioner's stopping rules and vertex-weight bound
+        cmaps = []
+        coarsen_to = max(30 * k, 256)
+        maxvw = max(1, 3 * n // (2 * coarsen_to))
+        counts = (C.c_int64 * 2)()
+        while levels[-1][0] > coarsen_to and len(levels) < 48:
+            ln, lm, lx, la, lw, lv = levels[-1]
+            cmap = torch.empty(ln, dtype=torch.int32, device=dev)
+            cx = torch.empty(ln + 1, dtype=torch.int64, device=dev)
+            ca = torch.empty(max(lm, 1), dtype=torch.int32, device=dev)
+            cw = torch.empty(max(lm, 1), dtype=torch.int32, device=dev)
+            cv = torch.empty(ln, dtype=torch.int32, device=dev)
+            ws = torch.empty(lib.ttg_kway_coarsen_workspace_bytes(ln, lm), dtype=torch.uint8, device=dev)
+            _ttg.check(lib.ttg_kway_coarsen(ln, lm, _ttg.ptr(lx), _ttg.ptr(la), _ttg.ptr(lw), _ttg.ptr(lv), maxvw,
+                                            int(seed), len(levels) - 1, _ttg.ptr(cmap), _ttg.ptr(cx), _ttg.ptr(ca),
+                                            _ttg.ptr(cw), _ttg.ptr(cv), counts, _ttg.ptr(ws), ws.numel(), stream),
+                       "kway_coarsen")
+            del ws
+            cn, cm = int(counts[0]), int(counts[1])
+            if cn > ln - ln // 20:   # the matching stalls (< 5 % fewer vertices)
+                break
+            cmaps.append(cmap)
+            levels.append((cn, cm, cx[:cn + 1].clone(), ca[:cm].clone(), cw[:cm].clone(), cv[:cn].clone()))
+        t2 = time.perf_counter()
+        times["coarsen_s"] = t2 - t1
+        # initial parts on the host: the host partitioner's grown trials and their refinement
+        cn, cm, cx, ca, cw, cv = levels[-1]
+        hx, ha, hw, hv = (np.ascontiguousarray(t.cpu().numpy()) for t in (cx, ca, cw, cv))
+        hpart = np.empty(cn, dtype=np.int32)
+        _ttg.check(lib.ttg_partition_kway_initial(cn, hx.ctypes.data, ha.ctypes.data if cm else None,
+                                                  hw.ctypes.data if cm else None, hv.ctypes.data, n, k, ub,
+                                                  int(seed), int(refine_passes), hpart.ctypes.data),
+                   "partition_kway_initial")
+        part = torch.from_numpy(hpart).to(dev)
+        t3 = time.perf_counter()
+        times["host_initial_s"] = t3 - t2
+        rstats = (C.c_int64 * 3)()
+        iterations = fills = 0
+        for lv in range(len(levels) - 1, -1, -1):
+            ln, lm, lx, la, lw, lvw = levels[lv]
+            if lv < len(levels) - 1:
+                fine = torch.empty(ln, dtype=torch.int32, device=dev)
+                cmap, coarse = cmaps[lv], part
+            else:
+                fine, cmap, coarse = part, None, None
+            ws = torch.empty(lib.ttg_kway_refine_workspace_bytes(ln, k), dtype=torch.uint8, device=dev)
+            _ttg.check(lib.ttg_kway_refine(ln, _ttg.ptr(lx), _ttg.ptr(la) if lm else None,
+                                           _ttg.ptr(lw) if lm else None, _ttg.ptr(lvw), n, k, ub, int(lv == 0),
+                                           int(seed), lv, int(refine_passes), _ttg.ptr(cmap), _ttg.ptr(coarse),
+                                           _ttg.ptr(fine), rstats, _ttg.ptr(ws), ws.numel(), stream), "kway_refine")
+            del ws
+            part = fine
+            iterations += int(rstats[0])
+            fills += int(rstats[2])
+            levels[lv] = None   # this level's graph is done with
+        sync()
+        t4 = time.perf_counter()
+        times["refine_s"] = t4 - t3
+        cut = C.c_int64(0)
+        if (return_cut or stats is not None) and nnz > 0:
+            ws = torch.empty(lib.ttg_kway_edge_cut_workspace_bytes(), dtype=torch.uint8, device=dev)
+            _ttg.check(lib.ttg_kway_edge_cut(n, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(part),
+                                             C.byref(cut), _ttg.ptr(ws), ws.numel(), stream), "kway_edge_cut")
+    if stats is not None:
+        stats.update(times, levels=len(cmaps) + 1, coarsest_nodes=cn, coarsest_edges=cm, sym_edges=m.value,
+                     refine_iterations=iterations, exact_fills=fills, cut=int(cut.value))
+    return (part, int(cut.value)) if return_cut else part
+
+
 def degree_permutation(g: CSRGraph, percentile: float = 80.0) -> torch.Tensor:
     """graphloader.py:275-285 (custom_reordering, is_degree=True): the nodes whose in-degree reaches the
     `percentile`-th percentile of all in-degrees first, the others behind them, both in increasing id."""
@@ -235,17 +359,25 @@ def reorder_graph(g: CSRGraph, algo: str, k: Optional[int] = None,
         if k is None:
             raise RuntimeError("reorder_graph('metis') needs k")
         perm = partition_permutation(kway_partition(g, k, seed=seed))
+    elif algo == "kway":
+        if k is None:
+            raise RuntimeError("reorder_graph('kway') needs k")
+        perm = partition_permutation(kway_partition_device(g, k, seed=seed))
     else:
         raise RuntimeError("reorder_graph: unknown algorithm %r" % algo)
     return permute_graph(g, perm), perm
 
 
-def recursive_metis_reorder(g: CSRGraph, partition_list, seed: int = 0) -> Tuple[CSRGraph, torch.Tensor]:
+def recursive_metis_reorder(g: CSRGraph, partition_list, seed: int = 0, algo: str = "metis"
+                            ) -> Tuple[CSRGraph, torch.Tensor]:
     """graphloader.py:358-372: one 'metis' reorder per entry of partition_list ([50, 60, 60] at
-    :432), each applied to the graph the previous one produced.  Returns the final graph and the
-    composed permutation (perm[i] = id in the ORIGINAL graph of final node i)."""
+    :432), each applied to the graph the previous one produced.  algo="kway" partitions on the device
+    instead.  Returns the final graph and the composed permutation (perm[i] = id in the ORIGINAL graph
+    of final node i)."""
+    if algo not in ("metis", "kway"):
+        raise RuntimeError("recursive_metis_reorder: unknown algorithm %r (metis or kway)" % algo)
     perm = torch.arange(g.num_nodes, dtype=torch.int64, device=g.indptr.device)
     for level, k in enumerate(partition_list):
-        g, p = reorder_graph(g, "metis", k=int(k), seed=seed + level)
+        g, p = reorder_graph(g, algo, k=int(k), seed=seed + level)
         perm = perm[p]
     return g, perm

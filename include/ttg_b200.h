@@ -453,6 +453,51 @@ int ttg_partition_kway(int64_t num_nodes, const int64_t* indptr, const int32_t* 
                        float ubfactor, uint64_t seed, int32_t refine_passes, int32_t* part_out,
                        int64_t* edge_cut_out);
 
+/* ttg_partition_kway_initial: the host partitioner's initial step on a weighted graph (host memory, CSR with
+ * edge weights adjw and vertex weights vw, both >= 1): eight grown partitions of the graph, each refined there with
+ * the coarse-level bounds of a `total_nodes`-node graph (1.3 x the bounds above), the one with the smallest cut in
+ * part_out [num_nodes].  The device partitioner below runs it on its coarsest level. */
+int ttg_partition_kway_initial(int64_t num_nodes, const int64_t* xadj, const int32_t* adj, const int32_t* adjw,
+                               const int32_t* vw, int64_t total_nodes, int32_t k, float ubfactor, uint64_t seed,
+                               int32_t refine_passes, int32_t* part_out);
+
+/* Multilevel k-way partition on the DEVICE (csrc/kway.cu): the scheme and the balance bounds of
+ * ttg_partition_kway with every data-parallel step on the GPU, driven level by level by the caller
+ * (reorder.kway_partition_device).  Not ttg_partition_kway's partition and not METIS'.  Deterministic in the seed.
+ * Every call runs on `stream` in the caller's workspace (its *_workspace_bytes query), allocates nothing, and
+ * refuses bad arguments before any CUDA call.  Weighted graphs are CSR: xadj int64 [n + 1], adj / adjw int32,
+ * vw int32 [n].
+ *   ttg_kway_symmetrise  the in-neighbour CSR (num_edges = indptr[num_nodes]) -> the undirected weighted graph
+ *                        (weight = directed edges between the pair, no self loops, unit vertex weights); adj and
+ *                        adjw hold 2 * num_edges entries, *sym_edges_out the used ones.  Ids out of range and an
+ *                        indptr that is not a CSR of num_edges are refused (checked on the device).
+ *   ttg_kway_coarsen     one level: matching (vertex weights <= maxvw; `level` varies the seed) and contraction.
+ *                        cmap [n]; cxadj [n + 1], cadj / cadjw [num_edges], cvw [n] hold the coarse graph;
+ *                        counts_out[0..1] = its vertex and edge counts (host memory; the call waits for them).
+ *   ttg_kway_refine      part [n] on this level: first projected from coarse_part through cmap (both NULL: part
+ *                        holds the labels already), then refined and rebalanced against the bounds of a
+ *                        total_nodes-node graph (finest != 0: the exact bounds, which the call guarantees there;
+ *                        else 1.3 x wider).  stats_out (host, may be NULL) [3]: label-propagation iterations,
+ *                        local rebalancing rounds, exact fills.
+ *   ttg_kway_edge_cut    *cut_out (host) = input edges whose ends lie in different parts. */
+size_t ttg_kway_symmetrise_workspace_bytes(int64_t num_nodes, int64_t num_edges);
+int ttg_kway_symmetrise(int64_t num_nodes, int64_t num_edges, const int64_t* indptr, const int32_t* indices,
+                        int64_t* xadj, int32_t* adj, int32_t* adjw, int32_t* vw, int64_t* sym_edges_out,
+                        void* workspace, size_t workspace_bytes, void* stream);
+size_t ttg_kway_coarsen_workspace_bytes(int64_t num_nodes, int64_t num_edges);
+int ttg_kway_coarsen(int64_t num_nodes, int64_t num_edges, const int64_t* xadj, const int32_t* adj,
+                     const int32_t* adjw, const int32_t* vw, int32_t maxvw, uint64_t seed, int32_t level,
+                     int32_t* cmap, int64_t* cxadj, int32_t* cadj, int32_t* cadjw, int32_t* cvw, int64_t* counts_out,
+                     void* workspace, size_t workspace_bytes, void* stream);
+size_t ttg_kway_refine_workspace_bytes(int64_t num_nodes, int32_t k);
+int ttg_kway_refine(int64_t num_nodes, const int64_t* xadj, const int32_t* adj, const int32_t* adjw,
+                    const int32_t* vw, int64_t total_nodes, int32_t k, float ubfactor, int32_t finest, uint64_t seed,
+                    int32_t level, int32_t refine_passes, const int32_t* cmap, const int32_t* coarse_part,
+                    int32_t* part, int64_t* stats_out, void* workspace, size_t workspace_bytes, void* stream);
+size_t ttg_kway_edge_cut_workspace_bytes(void);
+int ttg_kway_edge_cut(int64_t num_nodes, const int64_t* indptr, const int32_t* indices, const int32_t* part,
+                      int64_t* cut_out, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
