@@ -38,7 +38,7 @@
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
 
-#include "common.cuh"
+#include "graph.cuh"
 
 namespace ttg {
 namespace {
@@ -81,16 +81,6 @@ __device__ __forceinline__ int64_t warp_sum_i64(int64_t x) {
   return x;
 }
 
-__device__ __forceinline__ int64_t lower_bound_u64(const uint64_t* a, int64_t len, uint64_t x) {
-  int64_t lo = 0, hi = len;
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (a[mid] < x) lo = mid + 1;
-    else hi = mid;
-  }
-  return lo;
-}
-
 // ---- sorted (row, col) keys -> weighted CSR -----------------------------------------------------------------
 // keys are (row << colbits) | col, sorted, with the dropped entries (self pairs, keyed `drop`) last.  The first
 // entry of every run of equal keys is its head; pos = exclusive scan of the heads gives each run its slot.
@@ -118,7 +108,7 @@ run_reduce_kernel(int64_t items, uint64_t drop, const uint64_t* __restrict__ key
   atomicAdd(uw + slot, weights ? weights[i] : 1);
 }
 
-// row r's bounds by binary search over the m distinct keys; the column of every entry; rows > counts[0] idle
+// row r's bounds by binary search over the m distinct keys; rows > counts[0] idle
 __global__ void __launch_bounds__(256)
 csr_rows_kernel(int64_t max_rows, const int64_t* __restrict__ counts, int colbits, const uint64_t* __restrict__ ukeys,
                 int64_t* __restrict__ xadj) {
@@ -126,13 +116,6 @@ csr_rows_kernel(int64_t max_rows, const int64_t* __restrict__ counts, int colbit
   const int64_t rows = counts[0], m = counts[1];
   if (r > rows || r > max_rows) return;
   xadj[r] = r == rows ? m : lower_bound_u64(ukeys, m, (uint64_t)r << colbits);
-}
-
-__global__ void __launch_bounds__(256)
-csr_cols_kernel(const int64_t* __restrict__ counts, uint64_t colmask, const uint64_t* __restrict__ ukeys,
-                int32_t* __restrict__ adj) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < counts[1]) adj[i] = (int32_t)(ukeys[i] & colmask);
 }
 
 // ---- symmetrise ------------------------------------------------------------------------------------------------
@@ -143,8 +126,8 @@ sym_emit_kernel(int64_t n, int64_t nnz, int colbits, uint64_t drop, const int64_
   const int64_t v = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (v >= n) return;
-  const int64_t lo = __ldg(indptr + v), hi = __ldg(indptr + v + 1);
-  if (lo < 0 || hi < lo || hi > nnz || (v == 0 && lo != 0) || (v == n - 1 && hi != nnz)) {
+  int64_t lo, hi;
+  if (!csr_row(indptr, n, nnz, v, &lo, &hi)) {
     flags[0] = 1;
     return;
   }
@@ -631,7 +614,7 @@ cut_kernel(int64_t n, const int64_t* __restrict__ indptr, const int32_t* __restr
 }
 
 // ---- workspaces ---------------------------------------------------------------------------------------------
-struct SymWs {
+struct KwaySymWs {
   uint64_t *keys_a, *keys_b;
   int64_t* pos;
   int64_t* counts;   // [0] rows, [1] distinct pairs
@@ -640,8 +623,8 @@ struct SymWs {
   size_t cub_bytes, total;
 };
 
-SymWs carve_sym(void* ws, int64_t n, int64_t nnz) {
-  SymWs w;
+KwaySymWs carve_kway_sym(void* ws, int64_t n, int64_t nnz) {
+  KwaySymWs w;
   Carver c{ws};
   const int64_t items = 2 * nnz > 0 ? 2 * nnz : 1;
   w.keys_a = (uint64_t*)c.take(sizeof(uint64_t) * (size_t)items);
@@ -760,10 +743,6 @@ RefineWs carve_refine(void* ws, int64_t n, int32_t k) {
   return w;
 }
 
-bool nodes_in_range(int64_t n) { return n > 0 && n < ((int64_t)1 << 31) - 1; }
-bool edges_in_range(int64_t m) { return m >= 0 && m <= ((int64_t)1 << 40); }
-unsigned grid(int64_t threads, int block = 256) { return (unsigned)ceil_div(threads > 0 ? threads : 1, block); }
-
 // sorted (row, col) keys in keys (drop last) -> xadj / adj / adjw; counts[0] must hold the row count
 int keys_to_csr(int64_t items, int colbits, uint64_t drop, cub::DoubleBuffer<uint64_t>& dk, const int32_t* weights,
                 int64_t max_rows, int64_t* pos, int64_t* counts, void* cub_tmp, size_t cub_bytes, int64_t* xadj,
@@ -779,7 +758,7 @@ int keys_to_csr(int64_t items, int colbits, uint64_t drop, cub::DoubleBuffer<uin
   TTG_LAUNCH_CHECK();
   csr_rows_kernel<<<grid(max_rows + 1), 256, 0, stream>>>(max_rows, counts, colbits, ukeys, xadj);
   TTG_LAUNCH_CHECK();
-  csr_cols_kernel<<<grid(items), 256, 0, stream>>>(counts, (1ull << colbits) - 1, ukeys, adj);
+  key_cols_kernel<<<grid(items), 256, 0, stream>>>(counts + 1, (1ull << colbits) - 1, ukeys, adj);
   TTG_LAUNCH_CHECK();
   return TTG_OK;
 }
@@ -987,24 +966,21 @@ int Refine::fill_apply(int64_t c, const int32_t* grouped) {
 using namespace ttg;
 
 extern "C" size_t ttg_kway_symmetrise_workspace_bytes(int64_t num_nodes, int64_t num_edges) {
-  if (!nodes_in_range(num_nodes) || !edges_in_range(num_edges)) return 0;
-  return carve_sym(nullptr, num_nodes, num_edges).total;
+  if (!nodes_in_range(num_nodes, kKwayMaxNodes) || !edges_in_range(num_edges)) return 0;
+  return carve_kway_sym(nullptr, num_nodes, num_edges).total;
 }
 
 extern "C" int ttg_kway_symmetrise(int64_t num_nodes, int64_t num_edges, const int64_t* indptr, const int32_t* indices,
                                    int64_t* xadj, int32_t* adj, int32_t* adjw, int32_t* vw, int64_t* sym_edges_out,
                                    void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  TTG_CHECK_ARG(nodes_in_range(num_nodes), "kway_symmetrise: num_nodes=%lld out of range", (long long)num_nodes);
+  TTG_CHECK_ARG(nodes_in_range(num_nodes, kKwayMaxNodes), "kway_symmetrise: num_nodes=%lld out of range",
+                (long long)num_nodes);
   TTG_CHECK_ARG(edges_in_range(num_edges), "kway_symmetrise: num_edges=%lld out of range", (long long)num_edges);
   TTG_CHECK_ARG(indptr && (indices || num_edges == 0) && xadj && adj && adjw && vw && sym_edges_out,
                 "kway_symmetrise: null pointer");
-  SymWs w = carve_sym(workspace, num_nodes, num_edges);
-  if (!workspace || workspace_bytes < w.total) {
-    set_error("kway_symmetrise: workspace %zu bytes, need %zu for %lld nodes / %lld edges", workspace_bytes, w.total,
-              (long long)num_nodes, (long long)num_edges);
-    return TTG_ENOMEM;
-  }
+  KwaySymWs w = carve_kway_sym(workspace, num_nodes, num_edges);
+  TTG_RC(check_workspace("kway_symmetrise", workspace, workspace_bytes, w.total));
   const int64_t n = num_nodes, items = 2 * num_edges;
   const int colbits = std::max(1, bits_for((uint64_t)(n - 1)));
   const uint64_t drop = 1ull << (2 * colbits);
@@ -1037,7 +1013,7 @@ extern "C" int ttg_kway_symmetrise(int64_t num_nodes, int64_t num_edges, const i
 }
 
 extern "C" size_t ttg_kway_coarsen_workspace_bytes(int64_t num_nodes, int64_t num_edges) {
-  if (!nodes_in_range(num_nodes) || !edges_in_range(num_edges)) return 0;
+  if (!nodes_in_range(num_nodes, kKwayMaxNodes) || !edges_in_range(num_edges)) return 0;
   return carve_coarsen(nullptr, num_nodes, num_edges).total;
 }
 
@@ -1046,18 +1022,15 @@ extern "C" int ttg_kway_coarsen(int64_t num_nodes, int64_t num_edges, const int6
                                 int32_t* cmap, int64_t* cxadj, int32_t* cadj, int32_t* cadjw, int32_t* cvw,
                                 int64_t* counts_out, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  TTG_CHECK_ARG(nodes_in_range(num_nodes), "kway_coarsen: num_nodes=%lld out of range", (long long)num_nodes);
+  TTG_CHECK_ARG(nodes_in_range(num_nodes, kKwayMaxNodes), "kway_coarsen: num_nodes=%lld out of range",
+                (long long)num_nodes);
   TTG_CHECK_ARG(edges_in_range(num_edges), "kway_coarsen: num_edges=%lld out of range", (long long)num_edges);
   TTG_CHECK_ARG(maxvw >= 1, "kway_coarsen: maxvw=%d below 1", maxvw);
   TTG_CHECK_ARG(xadj && (num_edges == 0 || (adj && adjw)) && vw && cmap && cxadj && (num_edges == 0 || (cadj && cadjw)) &&
                     cvw && counts_out,
                 "kway_coarsen: null pointer");
   CoarsenWs w = carve_coarsen(workspace, num_nodes, num_edges);
-  if (!workspace || workspace_bytes < w.total) {
-    set_error("kway_coarsen: workspace %zu bytes, need %zu for %lld nodes / %lld edges", workspace_bytes, w.total,
-              (long long)num_nodes, (long long)num_edges);
-    return TTG_ENOMEM;
-  }
+  TTG_RC(check_workspace("kway_coarsen", workspace, workspace_bytes, w.total));
   const int64_t n = num_nodes, m = num_edges;
   const uint64_t lseed = mix64(seed ^ mix64(0x636f6172ull + (uint64_t)level));
   // handshake matching
@@ -1115,7 +1088,7 @@ extern "C" int ttg_kway_coarsen(int64_t num_nodes, int64_t num_edges, const int6
 }
 
 extern "C" size_t ttg_kway_refine_workspace_bytes(int64_t num_nodes, int32_t k) {
-  if (!nodes_in_range(num_nodes) || k < 1 || k > num_nodes) return 0;
+  if (!nodes_in_range(num_nodes, kKwayMaxNodes) || k < 1 || k > num_nodes) return 0;
   return carve_refine(nullptr, num_nodes, k).total;
 }
 
@@ -1125,17 +1098,13 @@ extern "C" int ttg_kway_refine(int64_t num_nodes, const int64_t* xadj, const int
                                const int32_t* coarse_part, int32_t* part, int64_t* stats_out, void* workspace,
                                size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  TTG_CHECK_ARG(nodes_in_range(num_nodes) && num_nodes <= total_nodes && total_nodes < (int64_t)INT32_MAX,
+  TTG_CHECK_ARG(nodes_in_range(num_nodes, total_nodes) && total_nodes <= kKwayMaxNodes,
                 "kway_refine: %lld of %lld nodes out of range", (long long)num_nodes, (long long)total_nodes);
   TTG_CHECK_ARG(k >= 1 && k <= num_nodes, "kway_refine: k=%d for %lld nodes", k, (long long)num_nodes);
   TTG_CHECK_ARG(ubfactor >= 1.0f, "kway_refine: ubfactor %g below 1", (double)ubfactor);
   TTG_CHECK_ARG(xadj && vw && part && (cmap == nullptr) == (coarse_part == nullptr), "kway_refine: null pointer");
   RefineWs ws = carve_refine(workspace, num_nodes, k);
-  if (!workspace || workspace_bytes < ws.total) {
-    set_error("kway_refine: workspace %zu bytes, need %zu for %lld nodes / k = %d", workspace_bytes, ws.total,
-              (long long)num_nodes, (long long)k);
-    return TTG_ENOMEM;
-  }
+  TTG_RC(check_workspace("kway_refine", workspace, workspace_bytes, ws.total));
   if (refine_passes <= 0) refine_passes = 10;
   KwayBounds kb;
   kway_bounds(total_nodes, k, ubfactor, &kb);
@@ -1212,12 +1181,10 @@ extern "C" size_t ttg_kway_edge_cut_workspace_bytes(void) { return 256; }
 extern "C" int ttg_kway_edge_cut(int64_t num_nodes, const int64_t* indptr, const int32_t* indices, const int32_t* part,
                                  int64_t* cut_out, void* workspace, size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  TTG_CHECK_ARG(nodes_in_range(num_nodes), "kway_edge_cut: num_nodes=%lld out of range", (long long)num_nodes);
+  TTG_CHECK_ARG(nodes_in_range(num_nodes, kKwayMaxNodes), "kway_edge_cut: num_nodes=%lld out of range",
+                (long long)num_nodes);
   TTG_CHECK_ARG(indptr && indices && part && cut_out, "kway_edge_cut: null pointer");
-  if (!workspace || workspace_bytes < 256) {
-    set_error("kway_edge_cut: workspace %zu bytes, need 256", workspace_bytes);
-    return TTG_ENOMEM;
-  }
+  TTG_RC(check_workspace("kway_edge_cut", workspace, workspace_bytes, 256));
   unsigned long long* cut = (unsigned long long*)workspace;
   TTG_CUDA(cudaMemsetAsync(cut, 0, sizeof(*cut), stream));
   cut_kernel<<<grid(num_nodes * 32), 256, 0, stream>>>(num_nodes, indptr, indices, part, cut);

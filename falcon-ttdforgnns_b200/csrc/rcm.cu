@@ -33,7 +33,7 @@
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 
-#include "common.cuh"
+#include "graph.cuh"
 
 namespace ttg {
 namespace {
@@ -50,8 +50,8 @@ sym_emit_kernel(int64_t n, int64_t nnz, int colbits, const int64_t* __restrict__
   const int64_t v = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (v >= n) return;
-  const int64_t lo = __ldg(indptr + v), hi = __ldg(indptr + v + 1);
-  if (hi < lo || hi > nnz || (v == 0 && lo != 0) || (v == n - 1 && hi != nnz)) {   // not a CSR of num_edges
+  int64_t lo, hi;
+  if (!csr_row(indptr, n, nnz, v, &lo, &hi)) {
     flags[1] = 1;
     return;
   }
@@ -67,16 +67,6 @@ sym_emit_kernel(int64_t n, int64_t nnz, int colbits, const int64_t* __restrict__
     vals[nnz + e] = kFromTranspose | (uint32_t)v;
     if (e + 1 < hi && __ldg(indices + e + 1) <= u) flags[0] = 1;   // not canonical
   }
-}
-
-__device__ __forceinline__ int64_t lower_bound_u64(const uint64_t* a, int64_t len, uint64_t x) {
-  int64_t lo = 0, hi = len;
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (a[mid] < x) lo = mid + 1;
-    else hi = mid;
-  }
-  return lo;
 }
 
 // row r of the distinct (row, col) keys, sorted: its bounds by binary search; degree = length + self loop
@@ -95,12 +85,6 @@ sym_rows_kernel(int64_t n, int64_t m, int colbits, const uint64_t* __restrict__ 
   const int64_t s = lower_bound_u64(ukeys + lo, hi - lo, self) + lo;
   sym_indptr[r] = lo;
   degree[r] = (int32_t)(hi - lo) + (s < hi && ukeys[s] == self ? 1 : 0);
-}
-
-__global__ void __launch_bounds__(256)
-sym_cols_kernel(int64_t m, uint64_t colmask, const uint64_t* __restrict__ ukeys, int32_t* __restrict__ out) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < m) out[i] = (int32_t)(ukeys[i] & colmask);
 }
 
 // general input: key (row, reverse appearance) for the per-row sort, value the column
@@ -294,7 +278,7 @@ order_reverse_kernel(int64_t n, const int32_t* __restrict__ sorted, int64_t* __r
 }
 
 // ---- workspaces ------------------------------------------------------------------------------------------
-struct SymWs {
+struct RcmSymWs {
   uint64_t *keys_a, *keys_b;
   uint32_t *vals_a, *vals_b;
   int64_t* num_unique;
@@ -303,8 +287,8 @@ struct SymWs {
   size_t cub_bytes, total;
 };
 
-SymWs carve_sym(void* ws, int64_t n, int64_t nnz) {
-  SymWs w;
+RcmSymWs carve_rcm_sym(void* ws, int64_t n, int64_t nnz) {
+  RcmSymWs w;
   Carver c{ws};
   const int64_t items = 2 * nnz > 0 ? 2 * nnz : 1;
   w.keys_a = (uint64_t*)c.take(sizeof(uint64_t) * (size_t)items);
@@ -368,10 +352,6 @@ OrderWs carve_order(void* ws, int64_t n) {
   return w;
 }
 
-bool nodes_in_range(int64_t n) { return n > 0 && n < ((int64_t)1 << 31); }
-// 2 * nnz (row, col) pairs; each in-list shorter than 2^31 (appearance ranks are 31-bit)
-bool edges_in_range(int64_t nnz) { return nnz >= 0 && nnz <= ((int64_t)1 << 40); }
-
 double ms_since(std::chrono::steady_clock::time_point t0) {
   return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
 }
@@ -383,7 +363,7 @@ using namespace ttg;
 
 extern "C" size_t ttg_rcm_symmetrise_workspace_bytes(int64_t num_nodes, int64_t num_edges) {
   if (!nodes_in_range(num_nodes) || !edges_in_range(num_edges)) return 0;
-  return carve_sym(nullptr, num_nodes, num_edges).total;
+  return carve_rcm_sym(nullptr, num_nodes, num_edges).total;
 }
 
 extern "C" int ttg_rcm_symmetrise(int64_t num_nodes, int64_t num_edges, const int64_t* indptr,
@@ -395,20 +375,16 @@ extern "C" int ttg_rcm_symmetrise(int64_t num_nodes, int64_t num_edges, const in
   TTG_CHECK_ARG(edges_in_range(num_edges), "rcm_symmetrise: num_edges=%lld out of range", (long long)num_edges);
   TTG_CHECK_ARG(indptr && (indices || num_edges == 0) && sym_indptr && sym_indices && degree && sym_edges_out,
                 "rcm_symmetrise: null pointer");
-  SymWs w = carve_sym(workspace, num_nodes, num_edges);
-  if (!workspace || workspace_bytes < w.total) {
-    set_error("rcm_symmetrise: workspace %zu bytes, need %zu for %lld nodes / %lld edges", workspace_bytes,
-              w.total, (long long)num_nodes, (long long)num_edges);
-    return TTG_ENOMEM;
-  }
+  RcmSymWs w = carve_rcm_sym(workspace, num_nodes, num_edges);
+  TTG_RC(check_workspace("rcm_symmetrise", workspace, workspace_bytes, w.total));
   const int colbits = bits_for((uint64_t)(num_nodes - 1));
   const int64_t items = 2 * num_edges;
   int64_t m = 0;
   int32_t flags[2] = {0, 0};
   TTG_CUDA(cudaMemsetAsync(w.flags, 0, 2 * sizeof(int32_t), stream));
   if (items > 0) {
-    sym_emit_kernel<<<(unsigned)ceil_div(num_nodes * 32, 256), 256, 0, stream>>>(
-        num_nodes, num_edges, colbits, indptr, indices, w.keys_a, w.vals_a, w.flags);
+    sym_emit_kernel<<<grid(num_nodes * 32), 256, 0, stream>>>(num_nodes, num_edges, colbits, indptr, indices,
+                                                              w.keys_a, w.vals_a, w.flags);
     TTG_LAUNCH_CHECK();
     cub::DoubleBuffer<uint64_t> dk(w.keys_a, w.keys_b);
     cub::DoubleBuffer<uint32_t> dv(w.vals_a, w.vals_b);
@@ -430,18 +406,15 @@ extern "C" int ttg_rcm_symmetrise(int64_t num_nodes, int64_t num_edges, const in
                 (long long)num_nodes);
       return TTG_EINVAL;
     }
-    sym_rows_kernel<<<(unsigned)ceil_div(num_nodes + 1, 256), 256, 0, stream>>>(num_nodes, m, colbits, ukeys,
-                                                                                  sym_indptr, degree);
+    sym_rows_kernel<<<grid(num_nodes + 1), 256, 0, stream>>>(num_nodes, m, colbits, ukeys, sym_indptr, degree);
     TTG_LAUNCH_CHECK();
     if (m > 0 && !flags[0]) {   // canonical: rows are the sorted distinct columns already
-      sym_cols_kernel<<<(unsigned)ceil_div(m, 256), 256, 0, stream>>>(m, (1ull << colbits) - 1, ukeys,
-                                                                       sym_indices);
+      key_cols_kernel<<<grid(m), 256, 0, stream>>>(w.num_unique, (1ull << colbits) - 1, ukeys, sym_indices);
       TTG_LAUNCH_CHECK();
     } else if (m > 0) {        // general: each row in reverse order of first appearance
       uint64_t* rkeys = dk.Current();
       uint32_t* rcols = dv.Current();
-      sym_reverse_key_kernel<<<(unsigned)ceil_div(m, 256), 256, 0, stream>>>(m, colbits, ukeys, uvals, rkeys,
-                                                                              rcols);
+      sym_reverse_key_kernel<<<grid(m), 256, 0, stream>>>(m, colbits, ukeys, uvals, rkeys, rcols);
       TTG_LAUNCH_CHECK();
       cub::DoubleBuffer<uint64_t> rk(rkeys, ukeys);
       cub::DoubleBuffer<uint32_t> rv(rcols, uvals);
@@ -470,18 +443,14 @@ extern "C" int ttg_rcm_order(int64_t num_nodes, int64_t sym_edges, const int64_t
                              size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   TTG_CHECK_ARG(nodes_in_range(num_nodes), "rcm_order: num_nodes=%lld out of range", (long long)num_nodes);
-  TTG_CHECK_ARG(sym_edges >= 0 && sym_edges <= 2 * ((int64_t)1 << 40), "rcm_order: sym_edges=%lld out of range",
+  TTG_CHECK_ARG(sym_edges >= 0 && sym_edges <= 2 * kMaxEdges, "rcm_order: sym_edges=%lld out of range",
                 (long long)sym_edges);
   TTG_CHECK_ARG(sym_indptr && (sym_indices || sym_edges == 0) && degree && rank_nodes && perm,
                 "rcm_order: null pointer");
   OrderWs w = carve_order(workspace, num_nodes);
-  if (!workspace || workspace_bytes < w.total) {
-    set_error("rcm_order: workspace %zu bytes, need %zu for %lld nodes", workspace_bytes, w.total,
-              (long long)num_nodes);
-    return TTG_ENOMEM;
-  }
+  TTG_RC(check_workspace("rcm_order", workspace, workspace_bytes, w.total));
   const int64_t n = num_nodes;
-  const unsigned nb = (unsigned)ceil_div(n, 256);
+  const unsigned nb = grid(n);
   const auto t0 = std::chrono::steady_clock::now();
 
   // components: converged label = rank of the component's seed
@@ -503,8 +472,7 @@ extern "C" int ttg_rcm_order(int64_t num_nodes, int64_t sym_edges, const int64_t
   if (sym_edges > 0) {
     for (int32_t changed = 1; changed;) {
       TTG_CUDA(cudaMemsetAsync(w.flags, 0, sizeof(int32_t), stream));
-      cc_hook_kernel<<<(unsigned)ceil_div(n * 32, 256), 256, 0, stream>>>(n, sym_indptr, sym_indices, w.node_of,
-                                                                          w.label, w.flags);
+      cc_hook_kernel<<<grid(n * 32), 256, 0, stream>>>(n, sym_indptr, sym_indices, w.node_of, w.label, w.flags);
       TTG_LAUNCH_CHECK();
       cc_jump_kernel<<<nb, 256, 0, stream>>>(n, w.node_of, w.label);
       TTG_LAUNCH_CHECK();
@@ -521,12 +489,12 @@ extern "C" int ttg_rcm_order(int64_t num_nodes, int64_t sym_edges, const int64_t
   TTG_RC(read_back(&components, w.flags + 1, stream));
   int64_t front = 0, m = components, pos = components, levels = 1;
   while (m > 0 && sym_edges > 0) {
-    const unsigned wb = (unsigned)ceil_div(m * 32, 256);
+    const unsigned wb = grid(m * 32);
     bfs_elect_kernel<<<wb, 256, 0, stream>>>(m, w.order + front, sym_indptr, sym_indices, w.visited,
                                              (unsigned long long*)w.owner);
     TTG_LAUNCH_CHECK();
-    bfs_count_kernel<<<(unsigned)ceil_div((m + 1) * 32, 256), 256, 0, stream>>>(
-        m, w.order + front, sym_indptr, sym_indices, w.visited, w.owner, w.cnt);
+    bfs_count_kernel<<<grid((m + 1) * 32), 256, 0, stream>>>(m, w.order + front, sym_indptr, sym_indices, w.visited,
+                                                             w.owner, w.cnt);
     TTG_LAUNCH_CHECK();
     size_t bytes = w.cub_bytes;
     TTG_CUDA(cub::DeviceScan::ExclusiveSum(w.cub_tmp, bytes, (const int32_t*)w.cnt, w.off, m + 1, stream));

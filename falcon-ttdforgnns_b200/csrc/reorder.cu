@@ -18,11 +18,14 @@
 //             (reorder_graph(g, "rcmk", backend="device")).
 #include <cub/device/device_scan.cuh>
 
-#include "common.cuh"
+#include "graph.cuh"
 
 namespace ttg {
 namespace {
 
+constexpr int32_t kBadPerm = 1, kBadGraph = 2;   // the bits of bad_flag (ttg_b200.h)
+
+// new row i = old row perm[i]: its length, checked, and inv[perm[i]] = i
 __global__ void __launch_bounds__(256)
 perm_degree_kernel(int64_t n, const int64_t* __restrict__ indptr, const int64_t* __restrict__ perm,
                    int64_t* __restrict__ inv, int64_t* __restrict__ deg, int32_t* __restrict__ bad) {
@@ -34,28 +37,36 @@ perm_degree_kernel(int64_t n, const int64_t* __restrict__ indptr, const int64_t*
   }
   const int64_t old = __ldg(perm + i);
   if (old < 0 || old >= n) {
-    atomicExch(bad, 1);
+    atomicOr(bad, kBadPerm);
     deg[i] = 0;
     return;
   }
   inv[old] = i;
-  deg[i] = __ldg(indptr + old + 1) - __ldg(indptr + old);
+  int64_t lo, hi;
+  const bool ok = csr_row(indptr, n, __ldg(indptr + n), old, &lo, &hi);
+  if (!ok) atomicOr(bad, kBadGraph);
+  deg[i] = ok ? hi - lo : 0;
 }
 
 // one warp per new row
 __global__ void __launch_bounds__(256)
 perm_fill_kernel(int64_t n, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
                  const int64_t* __restrict__ perm, const int64_t* __restrict__ inv,
-                 const int64_t* __restrict__ new_indptr, int32_t* __restrict__ new_indices,
-                 const int32_t* __restrict__ bad) {
+                 const int64_t* __restrict__ new_indptr, int32_t* __restrict__ new_indices, int32_t* bad) {
   const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
-  if (row >= n || *bad) return;
+  if (row >= n || *bad) return;   // every row read below passed perm_degree_kernel's checks
   const int64_t old = __ldg(perm + row);
   const int64_t src = __ldg(indptr + old), cnt = __ldg(indptr + old + 1) - src;
   const int64_t dst = __ldg(new_indptr + row);
-  for (int64_t j = lane; j < cnt; j += 32)
-    new_indices[dst + j] = (int32_t)__ldg(inv + __ldg(indices + src + j));
+  bool out = false;   // an id outside [0, n): reported once after the loop, which stays free of atomics
+  for (int64_t j = lane; j < cnt; j += 32) {
+    const int32_t u = __ldg(indices + src + j);
+    const bool in = u >= 0 && u < n;
+    out |= !in;
+    new_indices[dst + j] = (int32_t)__ldg(inv + (in ? u : 0));
+  }
+  if (out) atomicOr(bad, kBadGraph);
 }
 
 __global__ void __launch_bounds__(256)
@@ -114,25 +125,20 @@ struct PermWs {
 };
 PermWs carve_perm(void* ws, int64_t n) {
   PermWs w;
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    char* p = ws ? (char*)ws + off : nullptr;
-    off += align_up(bytes, 256);
-    return (void*)p;
-  };
-  w.inv = (int64_t*)take(sizeof(int64_t) * (size_t)n);
-  w.deg = (int64_t*)take(sizeof(int64_t) * (size_t)(n + 1));
-  w.bad = (int32_t*)take(sizeof(int32_t));
+  Carver c{ws};
+  w.inv = (int64_t*)c.take(sizeof(int64_t) * (size_t)n);
+  w.deg = (int64_t*)c.take(sizeof(int64_t) * (size_t)(n + 1));
+  w.bad = (int32_t*)c.take(sizeof(int32_t));
   w.cub_bytes = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, w.cub_bytes, (const int64_t*)nullptr, (int64_t*)nullptr, (int)(n + 1));
-  w.cub_tmp = take(w.cub_bytes);
-  w.total = off;
+  w.cub_tmp = c.take(w.cub_bytes);
+  w.total = c.off;
   return w;
 }
 }  // namespace
 
 extern "C" size_t ttg_permute_csr_workspace_bytes(int64_t num_nodes) {
-  if (num_nodes <= 0 || num_nodes >= (int64_t)1 << 31) return 0;
+  if (!nodes_in_range(num_nodes)) return 0;
   return carve_perm(nullptr, num_nodes).total;
 }
 
@@ -141,25 +147,20 @@ extern "C" int ttg_permute_csr(int64_t num_nodes, const int64_t* indptr, const i
                                int64_t* inverse_out, int32_t* bad_flag, void* workspace,
                                size_t workspace_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  TTG_CHECK_ARG(num_nodes > 0 && num_nodes < (int64_t)1 << 31, "permute_csr: num_nodes=%lld out of range",
-                (long long)num_nodes);
+  TTG_CHECK_ARG(nodes_in_range(num_nodes), "permute_csr: num_nodes=%lld out of range", (long long)num_nodes);
   TTG_CHECK_ARG(indptr && perm && new_indptr && bad_flag, "permute_csr: null pointer");
   PermWs w = carve_perm(workspace, num_nodes);
-  if (!workspace || workspace_bytes < w.total) {
-    set_error("permute_csr: workspace %zu bytes, need %zu", workspace_bytes, w.total);
-    return TTG_ENOMEM;
-  }
+  TTG_RC(check_workspace("permute_csr", workspace, workspace_bytes, w.total));
   int64_t* inv = inverse_out ? inverse_out : w.inv;
   TTG_CUDA(cudaMemsetAsync(bad_flag, 0, sizeof(int32_t), stream));
-  perm_degree_kernel<<<(unsigned)ceil_div(num_nodes + 1, 256), 256, 0, stream>>>(num_nodes, indptr, perm,
-                                                                                   inv, w.deg, bad_flag);
+  perm_degree_kernel<<<grid(num_nodes + 1), 256, 0, stream>>>(num_nodes, indptr, perm, inv, w.deg, bad_flag);
   TTG_LAUNCH_CHECK();
   size_t bytes = w.cub_bytes;
   TTG_CUDA(cub::DeviceScan::ExclusiveSum(w.cub_tmp, bytes, (const int64_t*)w.deg, new_indptr,
                                          (int)(num_nodes + 1), stream));
   count_launch();
-  perm_fill_kernel<<<(unsigned)ceil_div(num_nodes * 32, 256), 256, 0, stream>>>(
-      num_nodes, indptr, indices, perm, inv, new_indptr, new_indices, bad_flag);
+  perm_fill_kernel<<<grid(num_nodes * 32), 256, 0, stream>>>(num_nodes, indptr, indices, perm, inv, new_indptr,
+                                                             new_indices, bad_flag);
   TTG_LAUNCH_CHECK();
   return TTG_OK;
 }
@@ -178,15 +179,15 @@ extern "C" int ttg_partition_grow(int64_t num_nodes, const int64_t* indptr, cons
                 (long long)k * cap, (long long)num_nodes);
   TTG_CHECK_ARG(indptr && labels_a && labels_b && sizes && changed, "partition_grow: null pointer");
   if (seeds) {   // first call: start from the seeds; later calls (seeds == NULL) continue from labels_a
-    const unsigned nb = (unsigned)ceil_div(num_nodes > k ? num_nodes : k, 256);
+    const unsigned nb = grid(num_nodes > k ? num_nodes : k);
     grow_init_kernel<<<nb, 256, 0, stream>>>(num_nodes, k, seeds, labels_a, sizes);
     TTG_LAUNCH_CHECK();
-    grow_seed_kernel<<<(unsigned)ceil_div(k, 256), 256, 0, stream>>>(num_nodes, k, seeds, labels_a, sizes);
+    grow_seed_kernel<<<grid(k), 256, 0, stream>>>(num_nodes, k, seeds, labels_a, sizes);
     TTG_LAUNCH_CHECK();
   }
   TTG_CUDA(cudaMemsetAsync(changed, 0, sizeof(int32_t), stream));
   for (int s = 0; s < sweeps; ++s) {
-    grow_sweep_kernel<<<(unsigned)ceil_div(num_nodes, 256), 256, 0, stream>>>(
+    grow_sweep_kernel<<<grid(num_nodes), 256, 0, stream>>>(
         num_nodes, indptr, indices, cap, (s & 1) ? labels_b : labels_a, (s & 1) ? labels_a : labels_b,
         sizes, changed);
     TTG_LAUNCH_CHECK();

@@ -46,7 +46,31 @@ import torch
 import _ttg
 from sampler import CSRGraph
 
-_scratch = _ttg._Workspace()
+
+def _edge_count(g: CSRGraph, who: str) -> int:
+    """indptr[-1], the entries the in-lists use; refused when the indices array holds fewer"""
+    nnz = int(g.indptr[-1])
+    if nnz > g.num_edges:
+        raise RuntimeError("%s: indptr[-1] = %d > %d indices" % (who, nnz, g.num_edges))
+    return nnz
+
+
+def _workspace(dev, who: str, query, **sizes) -> torch.Tensor:
+    """A workspace of one call alone: the symmetrise ones take ~24 bytes per symmetrised entry (7 GB at products
+    shape), too much to keep for the process.  A size of 0 is the C side refusing `sizes` (in query order)."""
+    nbytes = query(*sizes.values())
+    if nbytes == 0:
+        raise RuntimeError("%s: %s out of range" % (who, " / ".join("%d %s" % (v, k) for k, v in sizes.items())))
+    return torch.empty(nbytes, dtype=torch.uint8, device=dev)
+
+
+def _check_k(who: str, k: int, n: int, ubfactor: float) -> int:
+    k = int(k)
+    if not 0 < k <= max(n, 1):
+        raise RuntimeError("%s: k=%d out of range" % (who, k))
+    if ubfactor < 1.0:
+        raise RuntimeError("%s: ubfactor %g below 1" % (who, ubfactor))
+    return k
 
 
 def inverse_permutation(perm: torch.Tensor) -> torch.Tensor:
@@ -64,20 +88,21 @@ def permute_graph(g: CSRGraph, perm: torch.Tensor) -> CSRGraph:
     dev = perm.device
     lib = _ttg.lib()
     with _ttg.on_device(dev):
+        _edge_count(g, "permute_graph")
         new_indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
         new_indices = torch.empty(max(g.num_edges, 1), dtype=torch.int32, device=dev)
         inv = torch.empty(n, dtype=torch.int64, device=dev)
         bad = torch.zeros(1, dtype=torch.int32, device=dev)
-        nbytes = lib.ttg_permute_csr_workspace_bytes(n)
-        if nbytes == 0:
-            raise RuntimeError("permute_graph: %d nodes out of range" % n)
-        ws = _scratch.get(dev, nbytes)
+        ws = _workspace(dev, "permute_graph", lib.ttg_permute_csr_workspace_bytes, nodes=n)
         rc = lib.ttg_permute_csr(n, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(perm),
                                  _ttg.ptr(new_indptr), _ttg.ptr(new_indices), _ttg.ptr(inv),
                                  _ttg.ptr(bad), _ttg.ptr(ws), ws.numel(), _ttg.stream_of(dev))
         _ttg.check(rc, "permute_csr")
+        flags = int(bad.item())   # bit 0: a perm id out of range, bit 1: a bad row or in-neighbour id
+        if flags == 2:
+            raise RuntimeError("permute_graph: the graph is not a CSR of %d nodes with ids in [0, %d)" % (n, n))
         # a permutation: every id in range (kernel) and every id hit once (inv o perm = id)
-        if int(bad.item()) or not bool((inv[perm] == torch.arange(n, device=dev)).all()):
+        if flags or not bool((inv[perm] == torch.arange(n, device=dev)).all()):
             raise RuntimeError("permute_graph: perm is not a permutation of 0..%d" % (n - 1))
     return CSRGraph(new_indptr, new_indices[:g.num_edges])
 
@@ -107,19 +132,12 @@ def _rcmk_device(g: CSRGraph, stats: Optional[dict]) -> torch.Tensor:
     lib = _ttg.lib()
     with _ttg.on_device(dev):
         t0 = time.perf_counter()
-        nnz = int(g.indptr[-1])
-        if nnz > g.num_edges:
-            raise RuntimeError("rcmk_permutation: indptr[-1] = %d > %d indices" % (nnz, g.num_edges))
+        nnz = _edge_count(g, "rcmk_permutation")
         sym_indptr = torch.empty(n + 1, dtype=torch.int64, device=dev)
         sym_indices = torch.empty(max(2 * nnz, 1), dtype=torch.int32, device=dev)
         degree = torch.empty(n, dtype=torch.int32, device=dev)
         sym_edges = C.c_int64(0)
-        nbytes = lib.ttg_rcm_symmetrise_workspace_bytes(n, nnz)
-        if nbytes == 0:
-            raise RuntimeError("rcmk_permutation: %d nodes / %d edges out of range" % (n, nnz))
-        # ~24 bytes per symmetrised entry (7 GB at products shape): a buffer of this call alone, not the
-        # module's scratch that lives as long as the process
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        ws = _workspace(dev, "rcmk_permutation", lib.ttg_rcm_symmetrise_workspace_bytes, nodes=n, edges=nnz)
         rc = lib.ttg_rcm_symmetrise(n, nnz, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(sym_indptr),
                                     _ttg.ptr(sym_indices), _ttg.ptr(degree), C.byref(sym_edges), _ttg.ptr(ws),
                                     ws.numel(), _ttg.stream_of(dev))
@@ -133,7 +151,7 @@ def _rcmk_device(g: CSRGraph, stats: Optional[dict]) -> torch.Tensor:
         perm = torch.empty(n, dtype=torch.int64, device=dev)
         counts = (C.c_int64 * 2)()
         phase_ms = (C.c_double * 3)()
-        ws = torch.empty(lib.ttg_rcm_order_workspace_bytes(n), dtype=torch.uint8, device=dev)
+        ws = _workspace(dev, "rcmk_permutation", lib.ttg_rcm_order_workspace_bytes, nodes=n)
         rc = lib.ttg_rcm_order(n, sym_edges.value, _ttg.ptr(sym_indptr), _ttg.ptr(sym_indices), _ttg.ptr(degree),
                                _ttg.ptr(rank_nodes), _ttg.ptr(perm), counts, phase_ms, _ttg.ptr(ws), ws.numel(),
                                _ttg.stream_of(dev))
@@ -186,9 +204,7 @@ def kway_partition(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int = 0, r
     most ubfactor * ceil(N / k) nodes.  The graph is copied to the host and the labels come back
     on the graph's device.  With return_cut also the number of edges between different parts."""
     n, dev = g.num_nodes, g.indptr.device
-    k = int(k)
-    if not 0 < k <= max(n, 1):
-        raise RuntimeError("kway_partition: k=%d out of range" % k)
+    k = _check_k("kway_partition", k, n, ubfactor)
     indptr = np.ascontiguousarray(g.indptr.cpu().numpy(), dtype=np.int64)
     indices = np.ascontiguousarray(g.indices.cpu().numpy()[:int(indptr[-1])], dtype=np.int32)
     part = np.empty(n, dtype=np.int32)
@@ -210,11 +226,7 @@ def kway_partition_device(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int
     initial parts of the coarsest graph are computed on the host, by the host partitioner's own code.  `stats`,
     when given, receives the seconds of each phase, the number of levels and the coarsest graph's size."""
     n, dev = g.num_nodes, g.indptr.device
-    k = int(k)
-    if not 0 < k <= max(n, 1):
-        raise RuntimeError("kway_partition_device: k=%d out of range" % k)
-    if ubfactor < 1.0:
-        raise RuntimeError("kway_partition_device: ubfactor %g below 1" % ubfactor)
+    k = _check_k("kway_partition_device", k, n, ubfactor)
     if n == 0 or k == 1:
         labels = torch.zeros(n, dtype=torch.int32, device=dev)
         return (labels, 0) if return_cut else labels
@@ -225,18 +237,13 @@ def kway_partition_device(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int
     with _ttg.on_device(dev):
         sync = torch.cuda.current_stream(dev).synchronize
         t0 = time.perf_counter()
-        nnz = int(g.indptr[-1])
-        if nnz > g.num_edges:
-            raise RuntimeError("kway_partition_device: indptr[-1] = %d > %d indices" % (nnz, g.num_edges))
-        nbytes = lib.ttg_kway_symmetrise_workspace_bytes(n, nnz)
-        if nbytes == 0:
-            raise RuntimeError("kway_partition_device: %d nodes / %d edges out of range" % (n, nnz))
+        nnz = _edge_count(g, "kway_partition_device")
         xadj = torch.empty(n + 1, dtype=torch.int64, device=dev)
         adj = torch.empty(max(2 * nnz, 1), dtype=torch.int32, device=dev)
         adjw = torch.empty(max(2 * nnz, 1), dtype=torch.int32, device=dev)
         vw = torch.empty(n, dtype=torch.int32, device=dev)
         m = C.c_int64(0)
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)   # ~24 bytes per symmetrised entry: this call's alone
+        ws = _workspace(dev, "kway_partition_device", lib.ttg_kway_symmetrise_workspace_bytes, nodes=n, edges=nnz)
         _ttg.check(lib.ttg_kway_symmetrise(n, nnz, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(xadj),
                                            _ttg.ptr(adj), _ttg.ptr(adjw), _ttg.ptr(vw), C.byref(m), _ttg.ptr(ws),
                                            ws.numel(), stream), "kway_symmetrise")
@@ -258,7 +265,7 @@ def kway_partition_device(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int
             ca = torch.empty(max(lm, 1), dtype=torch.int32, device=dev)
             cw = torch.empty(max(lm, 1), dtype=torch.int32, device=dev)
             cv = torch.empty(ln, dtype=torch.int32, device=dev)
-            ws = torch.empty(lib.ttg_kway_coarsen_workspace_bytes(ln, lm), dtype=torch.uint8, device=dev)
+            ws = _workspace(dev, "kway_partition_device", lib.ttg_kway_coarsen_workspace_bytes, nodes=ln, edges=lm)
             _ttg.check(lib.ttg_kway_coarsen(ln, lm, _ttg.ptr(lx), _ttg.ptr(la), _ttg.ptr(lw), _ttg.ptr(lv), maxvw,
                                             int(seed), len(levels) - 1, _ttg.ptr(cmap), _ttg.ptr(cx), _ttg.ptr(ca),
                                             _ttg.ptr(cw), _ttg.ptr(cv), counts, _ttg.ptr(ws), ws.numel(), stream),
@@ -291,7 +298,7 @@ def kway_partition_device(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int
                 cmap, coarse = cmaps[lv], part
             else:
                 fine, cmap, coarse = part, None, None
-            ws = torch.empty(lib.ttg_kway_refine_workspace_bytes(ln, k), dtype=torch.uint8, device=dev)
+            ws = _workspace(dev, "kway_partition_device", lib.ttg_kway_refine_workspace_bytes, nodes=ln, parts=k)
             _ttg.check(lib.ttg_kway_refine(ln, _ttg.ptr(lx), _ttg.ptr(la) if lm else None,
                                            _ttg.ptr(lw) if lm else None, _ttg.ptr(lvw), n, k, ub, int(lv == 0),
                                            int(seed), lv, int(refine_passes), _ttg.ptr(cmap), _ttg.ptr(coarse),
@@ -306,7 +313,7 @@ def kway_partition_device(g: CSRGraph, k: int, ubfactor: float = 1.03, seed: int
         times["refine_s"] = t4 - t3
         cut = C.c_int64(0)
         if (return_cut or stats is not None) and nnz > 0:
-            ws = torch.empty(lib.ttg_kway_edge_cut_workspace_bytes(), dtype=torch.uint8, device=dev)
+            ws = _workspace(dev, "kway_partition_device", lib.ttg_kway_edge_cut_workspace_bytes)
             _ttg.check(lib.ttg_kway_edge_cut(n, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(part),
                                              C.byref(cut), _ttg.ptr(ws), ws.numel(), stream), "kway_edge_cut")
     if stats is not None:
@@ -343,6 +350,8 @@ def reorder_graph(g: CSRGraph, algo: str, k: Optional[int] = None,
         raise RuntimeError("reorder_graph: unknown backend %r (host or device)" % backend)
     if backend != "host" and algo != "rcmk":
         raise RuntimeError("reorder_graph: backend=%r applies to 'rcmk' only, not %r" % (backend, algo))
+    if algo in ("grow", "metis", "kway") and k is None:
+        raise RuntimeError("reorder_graph(%r) needs k" % algo)
     if algo == "custom":
         if nodes_perm is None:
             raise RuntimeError("reorder_graph('custom') needs nodes_perm")
@@ -352,16 +361,10 @@ def reorder_graph(g: CSRGraph, algo: str, k: Optional[int] = None,
     elif algo == "degree":
         perm = degree_permutation(g)
     elif algo == "grow":
-        if k is None:
-            raise RuntimeError("reorder_graph('grow') needs k")
         perm = partition_permutation(grow_partition(g, k, seed=seed))
     elif algo == "metis":
-        if k is None:
-            raise RuntimeError("reorder_graph('metis') needs k")
         perm = partition_permutation(kway_partition(g, k, seed=seed))
     elif algo == "kway":
-        if k is None:
-            raise RuntimeError("reorder_graph('kway') needs k")
         perm = partition_permutation(kway_partition_device(g, k, seed=seed))
     else:
         raise RuntimeError("reorder_graph: unknown algorithm %r" % algo)

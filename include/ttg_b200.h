@@ -395,8 +395,11 @@ int ttg_sample_block(int64_t num_nodes, const int64_t* g_indptr, const int32_t* 
  *
  * ttg_permute_csr: the graph under the node permutation `perm` (new node i = old node perm[i],
  * DGL's nodes_perm convention); neighbour lists keep their order, ids are mapped through the
- * inverse permutation (also written to inverse_out when not NULL).  *bad_flag (device int32) is
- * set to 1 when perm holds an id outside [0, n); the outputs are then undefined.
+ * inverse permutation (also written to inverse_out when not NULL).  *bad_flag (device int32) has
+ * bit 0 set when perm holds an id outside [0, n), bit 1 when a row it reads is not a row of a CSR
+ * of indptr[n] entries (indptr[0] = 0, non-decreasing) or holds an id outside [0, n); the outputs
+ * are then undefined.  The caller makes sure that indices holds indptr[n] entries and that perm
+ * holds no id twice: a repeated id sets no bit, and its rows may overrun new_indices.
  *
  * ttg_partition_grow: k parts grown from `seeds` by capacity-bounded label propagation over the
  * in-neighbour lists -- the stand-in for METIS-k (NOT the same partition; connected parts of at

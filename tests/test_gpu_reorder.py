@@ -55,6 +55,27 @@ def test_permute_graph_rejects_non_permutations(ttg_lib):
             reorder.permute_graph(g, torch.tensor(bad, dtype=torch.int64, device=DEV))
 
 
+@pytest.mark.parametrize("fault", ["id_equal_to_n", "negative_id", "decreasing_indptr", "indptr0_not_zero",
+                                   "indptr_beyond_indices"])
+def test_permute_graph_refuses_a_bad_graph(ttg_lib, fault):
+    """Under a valid permutation the graph itself is checked, before any id is looked up or any row is copied."""
+    import reorder
+    indptr = np.array([0, 2, 3, 5], dtype=np.int64)
+    indices = np.array([1, 2, 0, 0, 1], dtype=np.int32)
+    if fault == "id_equal_to_n":
+        indices[2] = 3
+    elif fault == "negative_id":
+        indices[4] = -1
+    elif fault == "decreasing_indptr":
+        indptr[1] = 4
+    elif fault == "indptr0_not_zero":
+        indptr[0] = 1
+    else:
+        indptr[3] = 6
+    with pytest.raises(RuntimeError, match=r"graph is not a CSR|indptr\[-1\] = 6 > 5 indices"):
+        reorder.permute_graph(_to_graph(indptr, indices), torch.tensor([2, 0, 1], dtype=torch.int64, device=DEV))
+
+
 def test_rcmk_is_scipys_order_and_reduces_bandwidth(ttg_lib):
     import reorder
     from scipy import sparse
