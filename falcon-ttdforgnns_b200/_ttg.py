@@ -76,6 +76,8 @@ SIGNATURES = {
     "ttg_mean_agg_workspace_bytes": (_sz, [_i64, _i64, _i32]),
     "ttg_mean_agg_plan": (C.c_int, [_i64, _i64, _vp, _vp, _sz, _vp, _sz, _vp]),
     "ttg_mean_agg": (C.c_int, [_i64, _i64, _i32, _vp, _vp, _vp, _sz, _vp, _vp, _vp, _sz, _vp]),
+    "ttg_mean_agg_sharded": (C.c_int, [_i64, _i64, _i32, _vp, _vp, _vp, _sz, _i32, C.POINTER(C.c_int64), _vp,
+                                       _vp, _vp, _sz, _vp]),
     "ttg_edge_softmax_csr_fwd": (C.c_int, [_i64, _i32, _vp, _vp, _vp, _vp]),
     "ttg_edge_softmax_csr_bwd": (C.c_int, [_i64, _i32, _vp, _vp, _vp, _vp, _vp]),
     "ttg_head_spmm_csr_fwd": (C.c_int, [_i64, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),

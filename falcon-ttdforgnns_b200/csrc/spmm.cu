@@ -232,14 +232,48 @@ agg_scatter_kernel(int64_t n, const int64_t* __restrict__ indptr, const AggCount
   }
 }
 
+// Where the source rows live.  DenseRows: one array x [N][F] (ttg_mean_agg).  BlockRows: `world` row blocks,
+// block r holding the rows of nodes [lo[r], lo[r + 1]) as mapped on this device (own memory, or a peer GPU's
+// through NVLink; ttg_mean_agg_sharded).  The owner block of a row is found by compares against all eight
+// bounds, selects and no branch (constant indices only: a computed index into the parameter would copy it to
+// the stack); lo[i] = bounds[world] for i >= world, which no valid source id reaches.  kU: source rows loaded
+// per lane before any is summed.
+struct DenseRows {
+  static constexpr int kU = kAggU;
+  using Key = int32_t;
+  const float* x;
+  __device__ __forceinline__ Key key(int32_t s, int32_t) const { return s; }
+  __device__ __forceinline__ const float* row(Key k, int32_t F) const { return x + (int64_t)k * F; }
+};
+struct BlockRows {   // the key is the row's address, found once per edge by the lane that read its id
+  static constexpr int kU = kAggU;
+  using Key = unsigned long long;
+  const float* blk[TTG_MAX_PEERS];
+  int32_t lo[TTG_MAX_PEERS];
+  __device__ __forceinline__ Key key(int32_t s, int32_t F) const {
+    const float* b = blk[0];
+    int32_t first = 0;
+#pragma unroll
+    for (int i = 1; i < TTG_MAX_PEERS; ++i) {
+      const bool in = s >= lo[i];
+      b = in ? blk[i] : b;
+      first = in ? lo[i] : first;
+    }
+    return (Key)(uintptr_t)(b + (int64_t)(s - first) * F);
+  }
+  __device__ __forceinline__ const float* row(Key k, int32_t) const { return (const float*)(uintptr_t)k; }
+};
+
 // One warp per item.  The item's indices are read once per 32 edges (one per lane) and handed round by
-// shuffles; kAggU source rows are then loaded per lane and column before any is summed.  VEC: 16-byte
-// columns (F % 4 == 0), else scalar ones; C column groups of the warp per pass over the edges.
-template <int C, bool VEC>
+// shuffles; Rows::kU source rows are then loaded per lane and column before any is summed.  VEC: 16-byte
+// columns (F % 4 == 0), else scalar ones; C column groups of the warp per pass over the edges.  Every row is
+// summed in edge order whatever Rows is, so the sharded call gives the bits of the dense one.
+template <int C, bool VEC, class Rows>
 __global__ void __launch_bounds__(256)
 mean_agg_kernel(int64_t cap, int32_t F, const int64_t* __restrict__ indptr, const int32_t* __restrict__ indices,
-                const int64_t* __restrict__ header, const AggItem* __restrict__ items, const float* __restrict__ x,
+                const int64_t* __restrict__ header, const AggItem* __restrict__ items, const Rows src,
                 float* __restrict__ out, float* __restrict__ partial) {
+  constexpr int kU = Rows::kU;
   const int64_t it = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (it >= cap || it >= __ldg(header)) return;
@@ -270,13 +304,13 @@ mean_agg_kernel(int64_t cap, int32_t F, const int64_t* __restrict__ indptr, cons
     for (int c = 0; c < C; ++c) col[c] = d0 + (c * 32 + lane) * kLane;
     for (int64_t base = e0; base < e1; base += 32) {
       const int n = (int)min((int64_t)32, e1 - base);
-      const int32_t mine = lane < n ? __ldg(indices + base + lane) : 0;
+      const typename Rows::Key mine = src.key(lane < n ? __ldg(indices + base + lane) : 0, F);
       int j = 0;
-      for (; j + kAggU <= n; j += kAggU) {
-        float r[kAggU][C][kLane];
+      for (; j + kU <= n; j += kU) {
+        float r[kU][C][kLane];
 #pragma unroll
-        for (int u = 0; u < kAggU; ++u) {
-          const float* row = x + (int64_t)__shfl_sync(0xffffffffu, mine, j + u) * F;
+        for (int u = 0; u < kU; ++u) {
+          const float* row = src.row(__shfl_sync(0xffffffffu, mine, j + u), F);
 #pragma unroll
           for (int c = 0; c < C; ++c) {
             if (col[c] < F) {
@@ -293,14 +327,14 @@ mean_agg_kernel(int64_t cap, int32_t F, const int64_t* __restrict__ indptr, cons
           }
         }
 #pragma unroll
-        for (int u = 0; u < kAggU; ++u)
+        for (int u = 0; u < kU; ++u)
 #pragma unroll
           for (int c = 0; c < C; ++c)
 #pragma unroll
             for (int k = 0; k < kLane; ++k) acc[c][k] += r[u][c][k];
       }
       for (; j < n; ++j) {
-        const float* row = x + (int64_t)__shfl_sync(0xffffffffu, mine, j) * F;
+        const float* row = src.row(__shfl_sync(0xffffffffu, mine, j), F);
 #pragma unroll
         for (int c = 0; c < C; ++c) {
           if (col[c] < F) {
@@ -364,6 +398,36 @@ mean_agg_finalize_kernel(int64_t cap, int32_t F, const int64_t* __restrict__ ind
 bool agg_nodes_ok(int64_t n) { return n >= 0 && n < ((int64_t)1 << 31); }
 // partial-row numbers are int32: E / W + E / (W + 1) < 2^31
 bool agg_edges_ok(int64_t e) { return e >= 0 && e <= ((int64_t)1 << 37); }
+
+// the item pass and, for nodes of several items, the finalize pass; partial rows at the start of the workspace
+template <class Rows>
+int launch_mean_agg(int64_t num_nodes, int64_t num_edges, int32_t F, const int64_t* indptr, const int32_t* indices,
+                    const AggPlan& p, const Rows& src, bool vec, float* out, void* workspace, cudaStream_t stream) {
+  float* partial = (float*)align_up((size_t)workspace, 256);
+  const int64_t cap = agg_cap_items(num_nodes, num_edges);
+  const unsigned nb = (unsigned)ceil_div(cap * 32, 256);
+  if (vec && F <= 128) {
+    mean_agg_kernel<1, true><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, src, out, partial);
+  } else if (vec) {
+    mean_agg_kernel<2, true><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, src, out, partial);
+  } else if (F <= 32) {
+    mean_agg_kernel<1, false><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, src, out, partial);
+  } else {
+    mean_agg_kernel<2, false><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, src, out, partial);
+  }
+  TTG_LAUNCH_CHECK();
+  const int64_t cap_multi = agg_cap_multi(num_edges);
+  if (cap_multi > 0) {
+    const unsigned nf = (unsigned)ceil_div(cap_multi * 32, 256);
+    if (vec) {
+      mean_agg_finalize_kernel<true><<<nf, 256, 0, stream>>>(cap_multi, F, indptr, p.header, p.multi, partial, out);
+    } else {
+      mean_agg_finalize_kernel<false><<<nf, 256, 0, stream>>>(cap_multi, F, indptr, p.header, p.multi, partial, out);
+    }
+    TTG_LAUNCH_CHECK();
+  }
+  return TTG_OK;
+}
 
 }  // namespace
 }  // namespace ttg
@@ -433,31 +497,55 @@ extern "C" int ttg_mean_agg(int64_t num_nodes, int64_t num_edges, int32_t F, con
     return TTG_ENOMEM;
   }
   if (num_nodes == 0) return TTG_OK;
-  float* partial = (float*)align_up((size_t)workspace, 256);
   const bool vec = F % 4 == 0 && (((uintptr_t)x | (uintptr_t)out) & 15) == 0;
-  const int64_t cap = agg_cap_items(num_nodes, num_edges);
-  const unsigned nb = (unsigned)ceil_div(cap * 32, 256);
-  if (vec && F <= 128) {
-    mean_agg_kernel<1, true><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, x, out, partial);
-  } else if (vec) {
-    mean_agg_kernel<2, true><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, x, out, partial);
-  } else if (F <= 32) {
-    mean_agg_kernel<1, false><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, x, out, partial);
-  } else {
-    mean_agg_kernel<2, false><<<nb, 256, 0, stream>>>(cap, F, indptr, indices, p.header, p.items, x, out, partial);
-  }
-  TTG_LAUNCH_CHECK();
-  const int64_t cap_multi = agg_cap_multi(num_edges);
-  if (cap_multi > 0) {
-    const unsigned nf = (unsigned)ceil_div(cap_multi * 32, 256);
-    if (vec) {
-      mean_agg_finalize_kernel<true><<<nf, 256, 0, stream>>>(cap_multi, F, indptr, p.header, p.multi, partial, out);
-    } else {
-      mean_agg_finalize_kernel<false><<<nf, 256, 0, stream>>>(cap_multi, F, indptr, p.header, p.multi, partial, out);
+  return launch_mean_agg(num_nodes, num_edges, F, indptr, indices, p, DenseRows{x}, vec, out, workspace, stream);
+}
+
+extern "C" int ttg_mean_agg_sharded(int64_t num_dst, int64_t num_edges, int32_t F, const int64_t* indptr,
+                                    const int32_t* indices, const void* plan, size_t plan_bytes, int32_t world,
+                                    const int64_t* host_bounds, const float* const* host_x_blocks, float* out,
+                                    void* workspace, size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  TTG_CHECK_ARG(F > 0, "mean_agg_sharded: F=%d must be positive", F);
+  TTG_CHECK_ARG(agg_nodes_ok(num_dst), "mean_agg_sharded: num_dst=%lld out of range", (long long)num_dst);
+  TTG_CHECK_ARG(agg_edges_ok(num_edges), "mean_agg_sharded: num_edges=%lld out of range", (long long)num_edges);
+  TTG_CHECK_ARG(world >= 1 && world <= TTG_MAX_PEERS, "mean_agg_sharded: world=%d not in 1..%d", world,
+                TTG_MAX_PEERS);
+  TTG_CHECK_ARG(host_bounds && host_x_blocks, "mean_agg_sharded: null bounds or block array");
+  TTG_CHECK_ARG(host_bounds[0] == 0, "mean_agg_sharded: bounds[0]=%lld, need 0", (long long)host_bounds[0]);
+  // source ids are int32: every node id, bounds[world] included, fits one
+  TTG_CHECK_ARG(host_bounds[world] < ((int64_t)1 << 31), "mean_agg_sharded: bounds[%d]=%lld out of range", world,
+                (long long)host_bounds[world]);
+  BlockRows src;
+  memset(&src, 0, sizeof(src));
+  for (int r = 0; r < world; ++r) {
+    TTG_CHECK_ARG(host_bounds[r + 1] >= host_bounds[r], "mean_agg_sharded: bounds decrease at %d (%lld > %lld)",
+                  r + 1, (long long)host_bounds[r], (long long)host_bounds[r + 1]);
+    if (host_bounds[r + 1] > host_bounds[r]) {
+      TTG_CHECK_ARG(host_x_blocks[r] != nullptr, "mean_agg_sharded: null block %d for %lld rows", r,
+                    (long long)(host_bounds[r + 1] - host_bounds[r]));
+      TTG_CHECK_ARG(((uintptr_t)host_x_blocks[r] & 15) == 0, "mean_agg_sharded: block %d not 16-byte aligned", r);
     }
-    TTG_LAUNCH_CHECK();
+    src.blk[r] = host_x_blocks[r];
+    src.lo[r] = (int32_t)host_bounds[r];
   }
-  return TTG_OK;
+  for (int r = world; r < TTG_MAX_PEERS; ++r) src.lo[r] = (int32_t)host_bounds[world];
+  TTG_CHECK_ARG(indptr && (indices || num_edges == 0) && plan && (out || num_dst == 0),
+                "mean_agg_sharded: null pointer");
+  TTG_CHECK_ARG(((uintptr_t)plan & 15) == 0, "mean_agg_sharded: plan buffer not 16-byte aligned");
+  const AggPlan p = carve_agg_plan(const_cast<void*>(plan), num_dst, num_edges);
+  if (plan_bytes < p.total) {
+    set_error("mean_agg_sharded: plan buffer %zu bytes, need %zu", plan_bytes, p.total);
+    return TTG_ENOMEM;
+  }
+  const size_t need = ttg_mean_agg_workspace_bytes(num_dst, num_edges, F);
+  if (!workspace || workspace_bytes < need) {
+    set_error("mean_agg_sharded: workspace %zu bytes, need %zu", workspace_bytes, need);
+    return TTG_ENOMEM;
+  }
+  if (num_dst == 0) return TTG_OK;
+  const bool vec = F % 4 == 0 && ((uintptr_t)out & 15) == 0;
+  return launch_mean_agg(num_dst, num_edges, F, indptr, indices, p, src, vec, out, workspace, stream);
 }
 
 extern "C" int ttg_spmm_csr_fwd(int64_t num_dst, int32_t F, const int64_t* indptr,

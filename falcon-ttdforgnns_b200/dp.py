@@ -98,6 +98,71 @@ def apply_optimizer(tt_p_shapes, tt_q_shapes, tt_ranks, tt_cores: Sequence[torch
         _ttg.workspace.set_plan(dev, None)   # cores changed through raw pointers: the group table is stale
 
 
+def map_peer_buffers(nbytes: int, device, group=None, what: str = "map_peer_buffers"):
+    """One device buffer of `nbytes` per rank of `group`, every buffer mapped into every rank's address space
+    (CUDA IPC through ttg_peer_alloc / _export / _open): (own buffer, the peer buffers opened here, a ctypes
+    array of TTG_MAX_PEERS pointers with every rank's buffer as mapped here).  Collective, one process per GPU
+    of one node.  A failure on ONE rank becomes a failure on ALL of them: all_gather_object carries each
+    rank's error next to its handle, the open phase ends in an all-reduce(MIN) of an ok flag, and on
+    disagreement every rank frees what it holds and raises RuntimeError."""
+    import socket
+    world = dist.get_world_size(group)
+    rank = dist.get_rank(group)
+    if world > _ttg.TTG_MAX_PEERS:
+        raise RuntimeError("%s: at most %d ranks" % (what, _ttg.TTG_MAX_PEERS))
+    lib = _ttg.lib()
+    own_ptr, opened = None, []
+    ptrs = (C.c_void_p * _ttg.TTG_MAX_PEERS)()
+    err, handle = None, None
+    with torch.cuda.device(device):
+        own = C.c_void_p()
+        if lib.ttg_peer_alloc(nbytes, C.byref(own)) != 0:
+            err = "peer_alloc: " + _ttg.last_error()
+        else:
+            own_ptr = own.value
+            h = (C.c_ubyte * _ttg.PEER_HANDLE_BYTES)()
+            if lib.ttg_peer_export(own, h) != 0:
+                err = "peer_export: " + _ttg.last_error()
+            else:
+                handle = bytes(h)
+        mine = (socket.gethostname(), handle, err)
+        everyone = [None] * world
+        dist.all_gather_object(everyone, mine, group=group)
+        errs = [e[2] for e in everyone if e[2]]
+        if not errs and any(e[0] != mine[0] for e in everyone):
+            errs = ["the ranks are not on one node"]
+        if errs:
+            release_peer_buffers(own_ptr, opened)
+            raise RuntimeError("%s: %s" % (what, errs[0]))
+        ok = 1
+        for r, (_, h, _) in enumerate(everyone):
+            if r == rank:
+                ptrs[r] = own_ptr
+                continue
+            p = C.c_void_p()
+            buf = (C.c_ubyte * _ttg.PEER_HANDLE_BYTES).from_buffer_copy(h)
+            if lib.ttg_peer_open(buf, C.byref(p)) != 0:
+                ok, err = 0, "peer_open(rank %d): %s" % (r, _ttg.last_error())
+                break
+            ptrs[r] = p.value
+            opened.append(p.value)
+        flag = torch.tensor([ok], dtype=torch.int32, device=device)
+        dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=group)   # also: every buffer is mapped everywhere
+        if int(flag.item()) == 0:
+            release_peer_buffers(own_ptr, opened)
+            raise RuntimeError("%s: %s" % (what, err or "a peer could not map the buffers"))
+    return own_ptr, opened, ptrs
+
+
+def release_peer_buffers(own, opened) -> None:
+    """Undo map_peer_buffers on this rank: close the peer mappings, free the own buffer."""
+    lib = _ttg.lib()
+    for p in opened:
+        lib.ttg_peer_close(C.c_void_p(p))
+    if own is not None:
+        lib.ttg_peer_free(C.c_void_p(own))
+
+
 class PeerExchange:
     """The exchange step without NCCL: gradient slots that every GPU of the node has mapped, and
     one kernel per step that publishes this rank's gradients, waits for the peers, sums the copies
@@ -124,68 +189,16 @@ class PeerExchange:
         self.group = group
         self.world = dist.get_world_size(group)
         self.rank = dist.get_rank(group)
-        if self.world > _ttg.TTG_MAX_PEERS:
-            raise RuntimeError("PeerExchange: at most %d ranks" % _ttg.TTG_MAX_PEERS)
         self.device = cores[0].device
         self.sizes = [c.numel() for c in cores]
         self.total = sum(self.sizes)
         self.seg = (C.c_int64 * len(self.sizes))(*self.sizes)
-        lib = _ttg.lib()
-        self.nbytes = lib.ttg_peer_buffer_bytes(self.total)
-        self.own, self.opened = None, []
-        self.ptrs = (C.c_void_p * _ttg.TTG_MAX_PEERS)()
-        # Construction is collective; a failure on ONE rank must become a failure on ALL of them (a rank that
-        # fell back to NCCL alone would leave the others spinning in the exchange kernel).  Every phase ends in
-        # an agreement: all_gather_object carries this rank's error next to its handle, the open phase is
-        # followed by an all-reduce(MIN) of an ok flag; on disagreement every rank frees what it holds and raises.
-        import socket
-        err, handle = None, None
-        with torch.cuda.device(self.device):
-            own = C.c_void_p()
-            if lib.ttg_peer_alloc(self.nbytes, C.byref(own)) != 0:
-                err = "peer_alloc: " + _ttg.last_error()
-            else:
-                self.own = own.value
-                h = (C.c_ubyte * _ttg.PEER_HANDLE_BYTES)()
-                if lib.ttg_peer_export(own, h) != 0:
-                    err = "peer_export: " + _ttg.last_error()
-                else:
-                    handle = bytes(h)
-            mine = (socket.gethostname(), handle, err)
-            everyone = [None] * self.world
-            dist.all_gather_object(everyone, mine, group=group)
-            errs = [e[2] for e in everyone if e[2]]
-            if not errs and any(e[0] != mine[0] for e in everyone):
-                errs = ["the ranks are not on one node"]
-            if errs:
-                self._release()
-                raise RuntimeError("PeerExchange: " + errs[0])
-            ok = 1
-            for r, (_, h, _) in enumerate(everyone):
-                if r == self.rank:
-                    self.ptrs[r] = self.own
-                    continue
-                p = C.c_void_p()
-                buf = (C.c_ubyte * _ttg.PEER_HANDLE_BYTES).from_buffer_copy(h)
-                if lib.ttg_peer_open(buf, C.byref(p)) != 0:
-                    ok, err = 0, "peer_open(rank %d): %s" % (r, _ttg.last_error())
-                    break
-                self.ptrs[r] = p.value
-                self.opened.append(p.value)
-            flag = torch.tensor([ok], dtype=torch.int32, device=self.device)
-            dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=group)   # also: every buffer is mapped everywhere
-            if int(flag.item()) == 0:
-                self._release()
-                raise RuntimeError("PeerExchange: " + (err or "a peer could not map the exchange buffers"))
+        self.nbytes = _ttg.lib().ttg_peer_buffer_bytes(self.total)
+        self.own, self.opened, self.ptrs = map_peer_buffers(self.nbytes, self.device, group, "PeerExchange")
 
     def _release(self) -> None:
-        lib = _ttg.lib()
-        for p in self.opened:
-            lib.ttg_peer_close(C.c_void_p(p))
-        self.opened = []
-        if self.own is not None:
-            lib.ttg_peer_free(C.c_void_p(self.own))
-            self.own = None
+        release_peer_buffers(self.own, self.opened)
+        self.own, self.opened = None, []
 
     def step(self, d_cores: Sequence[torch.Tensor], tt_cores: Sequence[torch.Tensor],
              optimizer: str = "sgd", learning_rate: float = 0.0, eps: float = 1e-10,

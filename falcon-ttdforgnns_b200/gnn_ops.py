@@ -14,7 +14,7 @@ bias) stay in torch: they are library GEMMs, not part of the path.
 """
 import ctypes as C
 from dataclasses import dataclass
-from typing import Optional, Tuple
+from typing import Optional, Sequence, Tuple
 
 import torch
 from torch import nn
@@ -247,6 +247,36 @@ def aggregate_full(g, x: torch.Tensor) -> torch.Tensor:
         rc = lib.ttg_mean_agg(n, e, F, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(plan), plan.numel(),
                               _ttg.ptr(x), _ttg.ptr(out), _ttg.ptr(ws), ws_bytes, _ttg.stream_of(dev))
         _ttg.check(rc, "mean_agg")
+    return out
+
+
+def aggregate_sharded(g, bounds: Sequence[int], blocks: Sequence[int], F: int, out: torch.Tensor) -> torch.Tensor:
+    """aggregate_full for the destination nodes of one shard, the source rows split over row blocks
+    (ttg_mean_agg_sharded): g holds the shard's in-lists (int64 indptr [num_dst + 1], int32 indices with GLOBAL
+    source ids); block r is the device address (an int) of the rows of nodes [bounds[r], bounds[r + 1]), [rows][F]
+    fp32, as mapped on out's device -- a peer GPU's buffer or any allocation.  Writes out [num_dst, F] and returns
+    it; bit-identical to aggregate_full over the concatenated blocks."""
+    n, e = g.indptr.numel() - 1, g.indices.numel()
+    _ttg.require_cuda(out, "out", torch.float32)
+    if out.dim() != 2 or tuple(out.shape) != (n, F):
+        raise RuntimeError("aggregate_sharded: out must be [num_dst=%d, F=%d], got %s" % (n, F, tuple(out.shape)))
+    world = len(blocks)
+    if len(bounds) != world + 1 or not 1 <= world <= _ttg.TTG_MAX_PEERS:
+        raise RuntimeError("aggregate_sharded: %d blocks and %d bounds (need 1..%d blocks and one bound more)"
+                           % (world, len(bounds), _ttg.TTG_MAX_PEERS))
+    dev = out.device
+    lib = _ttg.lib()
+    ws_bytes = lib.ttg_mean_agg_workspace_bytes(n, e, F)
+    if ws_bytes == 0:
+        raise RuntimeError("aggregate_sharded: %d nodes / %d edges / F=%d out of range" % (n, e, F))
+    with _ttg.on_device(dev):
+        plan = mean_agg_plan(g)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        b = (C.c_int64 * (world + 1))(*[int(x) for x in bounds])
+        x = (C.c_void_p * world)(*[int(p) for p in blocks])
+        rc = lib.ttg_mean_agg_sharded(n, e, F, _ttg.ptr(g.indptr), _ttg.ptr(g.indices), _ttg.ptr(plan), plan.numel(),
+                                      world, b, x, _ttg.ptr(out), _ttg.ptr(ws), ws.numel(), _ttg.stream_of(dev))
+        _ttg.check(rc, "mean_agg_sharded")
     return out
 
 

@@ -12,7 +12,7 @@ from torch import nn
 
 import dp
 from FBTT.tt_embeddings_ops import OptimType, TTEmbeddingBag
-from gnn_ops import Block, SAGEConv
+from gnn_ops import Block, SAGEConv, mean_agg_plan
 from sampler import CSRGraph
 
 
@@ -139,6 +139,222 @@ def evaluate(model: SAGE, g: CSRGraph, labels: torch.Tensor, val_nid: torch.Tens
     val_acc = float(hit[val_nid.to(pred.device)].float().mean())
     test_acc = float(hit[test_nid.to(pred.device)].float().mean())
     return val_acc, test_acc, pred
+
+
+def shard_bounds(indptr: torch.Tensor, world: int) -> List[int]:
+    """world + 1 node ids splitting nodes 0 .. N - 1 into contiguous shards of about equal weight, a node
+    weighing deg(v) + ceil(E / N): bounds[r] is the first node whose prefix weight reaches r / world of the
+    total (a search on indptr, so every rank derives the same bounds).  Shards may be empty when world > N."""
+    n = indptr.numel() - 1
+    e = int(indptr[-1]) if n > 0 else 0
+    c = -(-e // max(n, 1))
+    total = e + n * c
+    prefix = indptr.to(torch.int64) + torch.arange(n + 1, dtype=torch.int64, device=indptr.device) * c
+    targets = torch.tensor([r * total // world for r in range(1, world)], dtype=torch.int64, device=indptr.device)
+    inner = torch.searchsorted(prefix, targets).tolist()
+    return [0] + [min(int(b), n) for b in inner] + [n]
+
+
+def check_bounds(bounds: Sequence[int], n: int, world: int) -> List[int]:
+    """Caller shard bounds as ints: world + 1 non-decreasing node ids from 0 to n, else ValueError."""
+    b = [int(x) for x in bounds]
+    if len(b) != world + 1:
+        raise ValueError("ShardedInference: %d bounds for %d ranks, need %d" % (len(b), world, world + 1))
+    if b[0] != 0 or b[-1] != n:
+        raise ValueError("ShardedInference: bounds must run from 0 to %d nodes, got %d .. %d" % (n, b[0], b[-1]))
+    if any(b[r + 1] < b[r] for r in range(world)):
+        raise ValueError("ShardedInference: bounds decrease: %s" % (b,))
+    return b
+
+
+class _DeviceRegion:
+    """A [rows, F] fp32 window of a peer buffer as a torch tensor (torch.as_tensor reads the interface and
+    shares the memory; the buffer outlives every view, see ShardedInference.close)."""
+
+    def __init__(self, ptr: int, rows: int, F: int):
+        self.__cuda_array_interface__ = {"shape": (rows, F), "typestr": "<f4", "data": (ptr, False),
+                                         "strides": None, "version": 2}
+
+
+class ShardedInference:
+    """SAGE.inference sharded over the GPUs of one node, one process per GPU (collective calls).  Rank r owns
+    nodes [bounds[r], bounds[r + 1]) and computes every layer for them only; the neighbour rows of other
+    shards are read straight from the peers' memory over NVLink (gnn_ops.aggregate_sharded on buffers mapped
+    by dp.map_peer_buffers), so no GPU holds a whole activation.
+
+        inf = ShardedInference(model, g)      # bounds=None: contiguous shards balanced by deg(v) + ceil(E / N)
+        logits = inf.inference()              # [hi - lo, n_classes]: model.inference(g)[lo:hi]
+        val_acc, test_acc = inf.evaluate(labels, val_nid, test_nid)    # the same numbers on every rank
+        inf.close()
+
+    Every rank holds the same graph and the same model (checked: a checksum of the dense layers and the cores
+    is compared across ranks, and every rank raises on a mismatch).  Caller bounds (e.g. the parts of
+    reorder_graph(g, "kway", world)) are taken as given.  Each rank's peer buffer holds its rows of the layer
+    input, the layer output and the projected input (fc_neigh first when a layer shrinks its rows), sized for
+    the widest layer.  Writes and remote reads of a region are ordered by a stream-ordered barrier (an
+    all-reduce of one element on the current stream), with no host synchronisation per layer.  The cores,
+    the parameters and model.training are left as they are."""
+
+    _IN, _OUT, _PROJ = 0, 1, 2
+
+    def __init__(self, model: SAGE, g: CSRGraph, group=None, bounds: Optional[Sequence[int]] = None):
+        import torch.distributed as dist
+        from gnn_ops import aggregate_sharded
+        if not (dist.is_available() and dist.is_initialized()):
+            raise RuntimeError("ShardedInference: torch.distributed is not initialised")
+        self._aggregate = aggregate_sharded
+        self.model, self.group = model, group
+        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
+        n = g.num_nodes
+        emb = model.embed_layer
+        if n > emb.num_embeddings:
+            raise RuntimeError("ShardedInference: the graph has %d nodes, the embedding %d rows"
+                               % (n, emb.num_embeddings))
+        self.bounds = shard_bounds(g.indptr, self.world) if bounds is None else check_bounds(bounds, n, self.world)
+        self.lo, self.hi = self.bounds[self.rank], self.bounds[self.rank + 1]
+        self.device = g.indptr.device
+        mine = _parameter_digest(model)
+        everyone = [None] * self.world
+        dist.all_gather_object(everyone, mine, group=group)
+        if any(d != everyone[0] for d in everyone):
+            raise RuntimeError("ShardedInference: the ranks hold different parameters (digests %s)"
+                               % ", ".join(d[:12] for d in everyone))
+        e0, e1 = (int(x) for x in g.indptr[[self.lo, self.hi]].tolist())
+        self.graph = CSRGraph(g.indptr[self.lo:self.hi + 1] - e0, g.indices[e0:e1])
+        mean_agg_plan(self.graph)                                    # built once, kept with the shard
+        self.width = max(max(l.in_feats, l.out_feats) for l in model.layers)
+        self.cap_rows = max(self.bounds[r + 1] - self.bounds[r] for r in range(self.world))
+        self.region_bytes = -(-max(self.cap_rows, 1) * self.width * 4 // 256) * 256
+        self.own, self.opened, self.ptrs = dp.map_peer_buffers(3 * self.region_bytes, self.device, group,
+                                                               "ShardedInference")
+        self.agg = torch.empty((self.hi - self.lo) * self.width, dtype=torch.float32, device=self.device)
+        self.token = torch.zeros(1, dtype=torch.float32, device=self.device)
+        self.reading = set()          # regions peers may still read: read by an aggregation since the last barrier
+        self.events = None            # a list: inference() appends (tag, recorded cuda.Event) at each phase
+
+    # ---- regions ------------------------------------------------------------------------------------------
+    def _blocks(self, region: int) -> List[int]:
+        return [self.ptrs[r] + region * self.region_bytes for r in range(self.world)]
+
+    def _own(self, region: int, F: int) -> torch.Tensor:
+        rows = self.hi - self.lo
+        if rows == 0:
+            return torch.empty((0, F), dtype=torch.float32, device=self.device)
+        return torch.as_tensor(_DeviceRegion(self.own + region * self.region_bytes, rows, F), device=self.device)
+
+    def _barrier(self) -> None:
+        if self.world > 1:
+            import torch.distributed as dist
+            dist.all_reduce(self.token, group=self.group)
+        self.reading.clear()
+
+    def _write(self, region: int) -> None:
+        """Before this rank overwrites `region`: no peer may still be reading it."""
+        if region in self.reading:
+            self._barrier()
+
+    def _mean(self, region: int, F: int) -> torch.Tensor:
+        """Neighbour mean of this shard over every rank's rows of `region` ([rows][F] each)."""
+        self._barrier()                                              # every rank's rows are written
+        self._mark("barrier")
+        rows = self.hi - self.lo
+        out = self.agg[:rows * F].view(rows, F)
+        self._aggregate(self.graph, self.bounds, self._blocks(region), F, out)
+        self.reading.add(region)
+        self._mark("aggregate")
+        return out
+
+    def _mark(self, tag: str) -> None:
+        if self.events is not None:
+            ev = torch.cuda.Event(enable_timing=True)
+            ev.record()
+            self.events.append((tag, ev))
+
+    def _own_rows(self) -> torch.Tensor:
+        """Layer-0 input of this shard: SAGE._all_rows restricted to nodes [lo, hi)."""
+        m, lo, rows = self.model, self.lo, self.hi - self.lo
+        emb = m.embed_layer
+        ids = torch.arange(lo, self.hi, device=self.device)
+        if m.embed_name == "eff":
+            return emb(ids)
+        h = emb.rows_range(lo, rows)
+        if h is not None:
+            return h
+        return emb(ids, torch.arange(rows + 1, device=self.device))
+
+    @torch.no_grad()
+    def inference(self) -> torch.Tensor:
+        """[hi - lo, n_classes] logits of this shard's nodes: the function model.inference(g)[lo:hi] computes,
+        in the operation order of SAGEConv.forward_full.  Collective."""
+        layers = self.model.layers
+        self._mark("start")
+        cur, nxt = self._IN, self._OUT
+        self._write(cur)
+        if self.hi > self.lo:
+            self._own(cur, layers[0].in_feats).copy_(self._own_rows())
+        self._mark("rows")
+        for l, layer in enumerate(layers):
+            x = self._own(cur, layer.in_feats)
+            if layer.in_feats > layer.out_feats:                    # fc_neigh before the mean
+                self._write(self._PROJ)
+                torch.mm(x, layer.fc_neigh.weight.t(), out=self._own(self._PROJ, layer.out_feats))
+                self._mark("gemm")
+                neigh = self._mean(self._PROJ, layer.out_feats)
+            else:
+                neigh = self._mean(cur, layer.in_feats)
+                neigh = torch.mm(neigh, layer.fc_neigh.weight.t())
+            self._write(nxt)
+            out = self._own(nxt, layer.out_feats)
+            torch.mm(x, layer.fc_self.weight.t(), out=out)
+            out += neigh
+            if layer.bias is not None:
+                out += layer.bias
+            if l != len(layers) - 1:
+                torch.relu_(out)
+            self._mark("gemm")
+            cur, nxt = nxt, cur
+        return self._own(cur, layers[-1].out_feats).clone()
+
+    @torch.no_grad()
+    def evaluate(self, labels: torch.Tensor, val_nid: torch.Tensor, test_nid: torch.Tensor):
+        """(validation accuracy, test accuracy) of the sharded inference, the same numbers on every rank and
+        the ones sage.evaluate computes: each rank marks the hits among its own nodes of each set, one
+        all-reduce assembles the hit vectors, and the accuracy is taken over them as sage.evaluate does."""
+        import torch.distributed as dist
+        pred = self.inference().argmax(1)
+        dev = self.device
+        own_hit = pred == labels[self.lo:self.hi].to(dev)
+        nids = [val_nid.to(dev), test_nid.to(dev)]
+        hits = []
+        for nid in nids:
+            inside = (nid >= self.lo) & (nid < self.hi)
+            h = torch.zeros(nid.numel(), dtype=torch.int32, device=dev)
+            h[inside] = own_hit[nid[inside] - self.lo].to(torch.int32)
+            hits.append(h)
+        flat = torch.cat(hits)
+        if self.world > 1:
+            dist.all_reduce(flat, group=self.group)
+        val_hit, test_hit = flat[:nids[0].numel()] != 0, flat[nids[0].numel():] != 0
+        return float(val_hit.float().mean()), float(test_hit.float().mean())
+
+    def close(self) -> None:
+        """Collective: frees this rank's buffer once no rank reads it any more."""
+        if self.own is None:
+            return
+        import torch.distributed as dist
+        torch.cuda.synchronize(self.device)
+        dist.barrier(group=self.group)
+        dp.release_peer_buffers(self.own, self.opened)
+        self.own, self.opened, self.agg = None, [], None
+
+
+def _parameter_digest(model: SAGE) -> str:
+    """sha256 of the dense layers and the TT cores, in a fixed order."""
+    import hashlib
+    h = hashlib.sha256()
+    for t in list(model.dense_parameters()) + list(model.embed_layer.tt_cores):
+        h.update(t.detach().contiguous().cpu().numpy().tobytes())
+    return h.hexdigest()
 
 
 def synthetic_graph(num_nodes: int, num_edges: int, device, seed: int = 0, alpha: float = 2.1

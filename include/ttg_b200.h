@@ -337,6 +337,24 @@ int ttg_mean_agg(int64_t num_nodes, int64_t num_edges, int32_t F, const int64_t*
                  const int32_t* indices, const void* plan, size_t plan_bytes, const float* x, float* out,
                  void* workspace, size_t workspace_bytes, void* stream);
 
+/* The same mean for the destination nodes of one shard, the source rows split over `world` row blocks (the
+ * GPUs of one node each holding the rows of a contiguous node range; sage.ShardedInference):
+ *   out[v][:] = (1 / deg(v)) * sum_{e in [indptr[v], indptr[v+1])} row(indices[e])[:],   v < num_dst
+ *   row(s) = host_x_blocks[r] + (s - bounds[r]) * F   for the r with bounds[r] <= s < bounds[r + 1].
+ * indptr int64 [num_dst + 1] and indices int32 [num_edges]: the shard's in-lists with GLOBAL source ids;
+ * plan: ttg_mean_agg_plan on this indptr (num_dst nodes); workspace: ttg_mean_agg_workspace_bytes(num_dst,
+ * num_edges, F).  host_bounds: world + 1 node ids, bounds[0] = 0, non-decreasing (empty blocks allowed),
+ * bounds[world] < 2^31; 1 <= world <= TTG_MAX_PEERS.  host_x_blocks[r]: block r as mapped on this device --
+ * its own allocation, a peer's through ttg_peer_open, or any device pointer --, 16-byte aligned, fp32
+ * [bounds[r + 1] - bounds[r]][F]; may be null for an empty block (and out for an empty shard).  The host checks these arguments before any
+ * CUDA call.  Every source id must be below bounds[world]: a precondition the device does not check.  The
+ * rows of every node are summed in edge order as in ttg_mean_agg, so out is bit-identical to ttg_mean_agg
+ * over the concatenated blocks. */
+int ttg_mean_agg_sharded(int64_t num_dst, int64_t num_edges, int32_t F, const int64_t* indptr,
+                         const int32_t* indices, const void* plan, size_t plan_bytes, int32_t world,
+                         const int64_t* host_bounds, const float* const* host_x_blocks, float* out,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------------------------
  * (f-4) the sparse part of GATConv on a CSR-by-destination block.
  * replaces: apply_edges(u_add_v) + leaky_relu + edge_softmax and update_all(u_mul_e, sum) of
